@@ -2,6 +2,7 @@
 """bench.py -- multivector products/s of the B200 batch evaluator (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one evaluation of the workload's expression over one full batch of
 synthetic random multivectors resident in HBM (one kernel launch).  The line says only
@@ -9,9 +10,11 @@ what THIS run measured:
 
 * headline (`value`, `roofline`): the workload of `--workload` (default cfg2 = BASELINE
   configs[1]), weak scaling under torchrun (every rank a full BASELINE batch, no
-  collective in the step).  The K-step timed loop is repeated until at least 0.5 s of
-  device time has passed; `ms_per_step` is the median over the repetitions of
-  (max over ranks of the repetition's CUDA-event time) / K.
+  collective in the step).  Exactly K steps are timed, after W warm-up steps (at least 3);
+  `ms_per_step` is (max over ranks of the CUDA-event time of the K steps) / K.  A short window
+  (the default K = 20 of cfg2 lasts ~16 ms) runs at burst clocks; the power-capped steady state
+  needs K steps to last >= 0.5 s (cfg2: K ~ 650).
+  `--dump-outputs DIR` writes what the last timed step computed (see dump_outputs).
 * `e2e`: the same metric through gaast_eval_host (pinned HOST arrays in and out, H2D +
   kernels + D2H in the timed region), run on EVERY rank at the same time between two
   barriers; value = elements of all ranks / the slowest rank's time.
@@ -41,7 +44,8 @@ if ROOT not in sys.path:
 
 METRIC = "multivector_products_per_sec"
 UNIT = "products/s"
-MIN_TIMED_SECONDS = 0.5  # the K-step loop is repeated until this much device time has passed
+FP64_SUSTAINED_SECONDS = 0.5  # length of the sustained live FP64-peak probe (gaast_diag_fp64_peak)
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much
 
 # stdout carries exactly ONE line, the JSON record.  Libraries print there too (NCCL announces its
 # version on stdout when the process group starts): file descriptor 1 is pointed at stderr for the
@@ -159,7 +163,7 @@ class ClockSampler:
         busy = [s for s, p in zip(sm, power) if p > 0.5 * max(power)] or sm
         return {"sm_mhz": statistics.median(busy), "sm_max_mhz": max(mx), "power_w_max": max(power),
                 "samples": len(sm), "samples_under_load": len(busy), "reasons": sorted(reasons),
-                "covers": "the headline workload's warm-up and timed repetitions (sampled every 50 ms)"}
+                "covers": "the headline workload's warm-up and timed steps (sampled every 50 ms)"}
 
 
 def _dist():
@@ -288,10 +292,12 @@ class Resident:
         self.engine = L.ENGINE_AUTO if engine is None else engine
         self.arith = L.ARITH_FMA if arith is None else arith
         self.counter = 0
+        self.last_set = None  # index into self.sets of the most recent step (or graph capture of one)
         self.comm = None
 
     def step(self):
-        _, s_in, s_out = self.sets[self.counter % self.n_sets]
+        self.last_set = self.counter % self.n_sets
+        _, s_in, s_out = self.sets[self.last_set]
         self.counter += 1
         if self.use_sum:
             self.plan.eval_sum(s_in, self.sums.data_ptr(), out=s_out, engine=self.engine, arith=self.arith)
@@ -307,9 +313,9 @@ class Resident:
 
 
 def timed(res, steps, warmup, torch, dist, world, allow_graph=True):
-    """Warm up, then repeat the K-step loop until MIN_TIMED_SECONDS of device time has passed.
-    Every repetition is bracketed by CUDA events on the ctx stream; barrier + synchronize on both
-    sides of the whole region; per repetition the MAX over ranks; returns the median ms per step."""
+    """Warm up, then time exactly `steps` steps, bracketed by CUDA events on the ctx stream, with a
+    barrier + synchronize on both sides; returns the MAX over ranks of that time, per step, and
+    `last_set`, the input/output set of the last timed step."""
     ctx = res.ctx
     dev = res.dev
     for _ in range(max(3, warmup)):
@@ -327,47 +333,37 @@ def timed(res, steps, warmup, torch, dist, world, allow_graph=True):
         with torch.cuda.graph(graph, stream=ctx.torch_stream):
             for _ in range(steps):
                 res.step()
+        graph.replay()  # untimed: the first launch of a graph also uploads it to the device
         torch.cuda.synchronize()
 
-    def one_rep(e0, e1):
-        e0.record()
-        if graph is not None:
-            graph.replay()
-        else:
-            for _ in range(steps):
-                res.step()
-        e1.record()
-
-    # calibration repetition (untimed): how many repetitions fill MIN_TIMED_SECONDS
-    c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    one_rep(c0, c1)
-    torch.cuda.synchronize()
-    cal_ms = max(c0.elapsed_time(c1), 1e-3)
-    reps = int(min(400, max(1, -(-MIN_TIMED_SECONDS * 1e3 // cal_ms))))
-    if world > 1:
-        t = torch.tensor([reps], dtype=torch.int64, device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        reps = int(t.item())
-    events = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(reps)]
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
     launches0 = ctx.launch_count
-    for e0, e1 in events:
-        one_rep(e0, e1)
+    # ~1 ms of device spin ahead of the window: the host enqueues the first steps meanwhile, so that the window holds
+    # the steps' device time and not the idle device waiting for the first launch after the synchronize
+    torch.cuda._sleep(2_000_000)
+    e0.record()
+    if graph is not None:
+        graph.replay()
+    else:
+        for _ in range(steps):
+            res.step()
+    e1.record()
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
+    last_set = res.last_set  # (a graph replays the steps of its capture: the last captured step's set)
     launches = ctx.launch_count - launches0  # this library's kernels only (NCCL's all-reduce kernel is not counted)
     if graph is not None:
-        launches = reps * steps * max(1, launches_per_step(res))
-    ms = torch.tensor([e0.elapsed_time(e1) for e0, e1 in events], dtype=torch.float64, device=dev)
+        launches = steps * max(1, launches_per_step(res))
+    ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:
-        dist.all_reduce(ms, op=dist.ReduceOp.MAX)  # per repetition, the slowest rank
-    ms = [float(x) for x in ms.tolist()]
-    return {"ms_per_step": statistics.median(ms) / steps, "ms_per_step_min": min(ms) / steps, "ms_per_step_first_rep": ms[0] / steps,
-            "ms_per_step_max": max(ms) / steps, "reps": reps, "timed_region_s": sum(ms) / 1e3,
-            "launches": launches, "cuda_graph": graph is not None}
+        dist.all_reduce(ms, op=dist.ReduceOp.MAX)  # the slowest rank
+    ms = float(ms.item())
+    return {"ms_per_step": ms / steps, "timed_region_s": ms / 1e3, "launches": launches, "cuda_graph": graph is not None,
+            "last_set": last_set}
 
 
 def launches_per_step(res):
@@ -377,6 +373,51 @@ def launches_per_step(res):
     res.step()
     res.torch.cuda.synchronize()
     return res.ctx.launch_count - c0
+
+
+def dump_columns(length, bytes_per_column, budget):
+    """Batch columns that --dump-outputs writes: None (all of them) when they fit in `budget` bytes, else a fixed,
+    seeded, sorted sample, the same for every run with the same batch length."""
+    import numpy as np
+    keep = max(1, budget // max(1, bytes_per_column))
+    if length <= keep:
+        return None
+    return np.sort(np.random.default_rng(0x6AA57D00).choice(length, size=keep, replace=False))
+
+
+class _GradeView:
+    """Grade k of a library-allocated batch ([rows][stride] in device memory) as a CUDA array interface, so that
+    torch.as_tensor sees it without a copy."""
+
+    def __init__(self, batch, k):
+        from gaast_b200 import _lib as L
+        size = 4 if batch.dtype == L.F32 else 8
+        self.__cuda_array_interface__ = {"shape": (batch.stored_rows(k), batch.length), "strides": (batch.stride * size, size),
+                                         "typestr": f"<f{size}", "data": (batch.grade_ptr(k), False), "version": 2}
+
+
+def dump_outputs(path, res, last_set):
+    """What the caller of the timed path received from its last step, as <path>/<name>.npy in the run's float type:
+    `out_g<k>` per root grade ([C(n,k), columns]) and, for a batch-sum plan, `sum` (the root vector).  When the
+    per-element outputs exceed DUMP_BYTES in all, the same seeded sample of columns (dump_columns) is taken of each
+    grade."""
+    import numpy as np
+    torch = res.torch
+    out = res.sets[last_set][2]
+    grades = res.plan.root_grades()
+    arrays = {f"out_g{k}": (out.tensors[k] if hasattr(out, "tensors") else torch.as_tensor(_GradeView(out, k), device=res.dev))
+              for k in grades}
+    whole = {"sum": res.sums} if res.use_sum else {}
+    per_column = sum(a.shape[0] * a.element_size() for a in arrays.values())
+    budget = DUMP_BYTES - sum(a.numel() * a.element_size() for a in whole.values()) - 1024 * (len(arrays) + len(whole))
+    cols = dump_columns(res.n, per_column, budget)
+    if cols is not None:
+        idx = torch.from_numpy(cols).to(res.dev)
+        arrays = {name: a.index_select(1, idx) for name, a in arrays.items()}
+    torch.cuda.synchronize()
+    os.makedirs(path, exist_ok=True)
+    for name, a in {**arrays, **whole}.items():
+        np.save(os.path.join(path, name + ".npy"), a.contiguous().cpu().numpy())
 
 
 def measure_e2e(res, steps, torch, dist, world, elements=None, host_mem="torch"):
@@ -454,11 +495,7 @@ def _workload_record(res, t, peak_gbs, w):
     kernel = res.kernel()
     traffic, traffic_src = _ncu_traffic(kernel, n) if not res.f32 else (None, "no capture of the f32 kernels")
     rec = {"elements_per_s": n / s, "products_per_s": n / s * w.products, "ms_per_step": t["ms_per_step"],
-           "ms_per_step_min": t["ms_per_step_min"], "ms_per_step_max": t["ms_per_step_max"],
-           # the first repetition starts on a GPU that has idled through the set-up: the burst figure, before the
-           # 1 kW power cap pulls the SM clock down (tools/power_probe.py); the median is the sustained one
-           "ms_per_step_first_rep": t["ms_per_step_first_rep"],
-           "timed_reps": t["reps"], "timed_region_s": t["timed_region_s"],
+           "timed_region_s": t["timed_region_s"],
            "hbm_gbs": n * res.bytes_per_elem / s / 1e9, "hbm_frac": n * res.bytes_per_elem / s / 1e9 / peak_gbs,
            "fp64_tflops": n * res.flops_per_elem / s / 1e12,
            "fp64_frac": n * res.flops_per_elem / s / 1e12 / FP64_PEAK_TFLOPS,
@@ -509,8 +546,7 @@ def run_cfg5_sharded(ctx, torch, dist, rank, world, steps, warmup, peak_gbs):
                               "nccl": "; transport: ncclAllReduce"}.get(res.comm.transport, "")
     t = timed(res, steps, warmup, torch, dist, world, allow_graph=False)
     s = t["ms_per_step"] / 1e3
-    rec.update({"ms_per_step": t["ms_per_step"], "ms_per_step_min": t["ms_per_step_min"], "timed_reps": t["reps"],
-                "timed_region_s": t["timed_region_s"], "shard_elements": res.n,
+    rec.update({"ms_per_step": t["ms_per_step"], "timed_region_s": t["timed_region_s"], "shard_elements": res.n,
                 "elements_per_s": total / s, "products_per_s": total / s * w.products,
                 "hbm_gbs_per_gpu": res.n * res.bytes_per_elem / s / 1e9,
                 "hbm_frac_per_gpu": res.n * res.bytes_per_elem / s / 1e9 / peak_gbs,
@@ -575,7 +611,8 @@ def run_gpu(args):
         batch = b1 - b0  # the BASELINE batch split into contiguous, 16-byte aligned slices
     # live FP64 FMA-pipe peak of THIS box (gaast_diag_fp64_peak: independent DFMA chains): a 20 ms burst on the idle
     # GPU, and -- measured after the headline, below -- 0.5 s sustained, the like-for-like denominator of a kernel
-    # that is itself timed over >= 0.5 s (an FP64-heavy B200 is power-capped well below 1965 MHz by then)
+    # timed over >= 0.5 s, i.e. with --steps large enough (an FP64-heavy B200 is power-capped well below 1965 MHz by
+    # then); the burst figure is the one to set beside a short timed window
     fp64_live = None
     if rank == 0 and not f32:
         try:
@@ -592,6 +629,8 @@ def run_gpu(args):
         res.comm = g.Comm.join(ctx, world, rank, uid[0])
     t = timed(res, args.steps, args.warmup, torch, dist, world)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, t["last_set"])
 
     n = res.n
     sec = t["ms_per_step"] / 1e3
@@ -612,9 +651,10 @@ def run_gpu(args):
                    + (" (+66-double NCCL all-reduce for the batch-sum, gaast_comm_allreduce_sum)" if res.comm is not None else ""),
                    "l2": f"inputs+outputs {n * res.bytes_per_elem / 1e9:.2f} GB per step (126 MB L2), "
                          f"{res.n_sets} input/output set(s) used in rotation",
-                   "timing": f"{t['reps']} repetitions of the {args.steps}-step loop ({t['timed_region_s']:.2f} s of device time), "
-                             f"median of per-repetition max-over-ranks CUDA-event times; min {t['ms_per_step_min']:.4f} "
-                             f"max {t['ms_per_step_max']:.4f} ms/step",
+                   "timing": f"{args.steps} timed steps ({t['timed_region_s']:.4f} s of device time), "
+                             f"max over ranks of their CUDA-event time"
+                             + ("; a window under 0.5 s runs at burst clocks" if t["timed_region_s"] < 0.5 else ""),
+                   "io_sets_rotated": res.n_sets,
                    "kernel": kernel, "cuda_graph": t["cuda_graph"]},
         "gpu_launches": t["launches"],
         "roofline": {"bound": "hbm", "achieved": gbs, "peak": peak_gbs, "unit": "GB/s", "frac": gbs / peak_gbs,
@@ -636,9 +676,9 @@ def run_gpu(args):
         try:
             if world > 1:
                 pass  # (rank 0 only measures while the other ranks wait at the next barrier)
-            fp64_live["sustained_tflops"] = ctx.fp64_peak(MIN_TIMED_SECONDS)
+            fp64_live["sustained_tflops"] = ctx.fp64_peak(FP64_SUSTAINED_SECONDS)
             fp64_live["how"] = ("gaast_diag_fp64_peak on this GPU in this run: 20 ms burst before the timed region, "
-                                f"{MIN_TIMED_SECONDS} s sustained after it")
+                                f"{FP64_SUSTAINED_SECONDS} s sustained after it")
         except Exception as ex:
             fp64_live["error"] = f"{type(ex).__name__}: {ex}"
     if fp64_live is not None:
@@ -807,7 +847,14 @@ def main():
     ap.add_argument("--all", action="store_true", default=True, help="also time the other BASELINE workloads (N=1)")
     ap.add_argument("--only", dest="all", action="store_false",
                     help="the headline workload only (no other_workloads, no cfg5_sharded)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload computed to DIR/<name>.npy (at most "
+                         "64 MB: a fixed, seeded sample of the batch columns when the outputs are larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "gaast_b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl gaast_b200)")
     if not args.all:
         args.no_sharded = True
     _claim_stdout()

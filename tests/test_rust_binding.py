@@ -148,9 +148,16 @@ def test_constants_match_the_header():
 
 
 def test_patches_apply_to_the_reference(tmp_path):
-    ref = "/root/reference"
+    """Needs a checkout of the reference (github.com/YPares/gaast), named by GAAST_REFERENCE_DIR.
+
+    The repository does not ship the reference.  To make this test self-contained, store the six files the patches
+    touch (Cargo.toml, src/ast/mod.rs, src/ast/specialize.rs, src/graded.rs, src/eval.rs, src/lib.rs) under
+    tests/golden/, use them when GAAST_REFERENCE_DIR is unset, and check each file's `git hash-object` against the
+    abbreviated pre-image blob id on the `index` line of the patch that touches it, so that the stored copies are
+    known to be the reference's own."""
+    ref = os.environ.get("GAAST_REFERENCE_DIR", "")
     if not os.path.isdir(os.path.join(ref, "src")):
-        pytest.skip("the reference checkout is not present here")
+        pytest.skip("GAAST_REFERENCE_DIR does not name a checkout of the reference")
     dst = tmp_path / "gaast"
     shutil.copytree(ref, dst, ignore=shutil.ignore_patterns(".git"))
     patches = sorted(os.path.join(PATCHES, p) for p in os.listdir(PATCHES) if p.endswith(".patch"))
