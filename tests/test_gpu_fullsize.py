@@ -103,7 +103,8 @@ def test_cfg5_vector_sandwich_preserves_the_bivector_norm_and_batch_sum():
     mag = (x * x).sum(0) + (y * y).sum(0)
     # conditioning: V.V >= 0.1 by construction; the inverse amplifies rounding by <= 12/0.1
     assert bool(((qx - qy).abs() <= 1e-9 * mag).all())
-    # fused batch-sum (tensor-memory accumulators) against a plain torch reduction of the stored result
+    # fused batch-sum (per-thread column sums in shared memory: the reflection lowering parks no rows, so the
+    # accumulators stay out of tensor memory) against a plain torch reduction of the stored result
     ref = out_t[2].sum(dim=1)
     scale = out_t[2].abs().sum(dim=1)
     assert bool(((sums - ref).abs() <= 1e-12 * scale).all())
