@@ -138,6 +138,10 @@ PROTOTYPES = {
     "gaast_batch_upload_f32": (C.c_int, vp, u32, vp, u64),
     "gaast_batch_download_f32": (C.c_int, vp, u32, vp, u64),
     "gaast_batch_zero": (C.c_int, vp),
+    "gaast_batch_pack_records": (C.c_int, vp, u64, u64, vp, u32),
+    "gaast_batch_unpack_records": (C.c_int, vp, u64, u64, vp, u32),
+    "gaast_batch_upload_records": (C.c_int, vp, u64, u64, vp, u32),
+    "gaast_batch_download_records": (C.c_int, vp, u64, u64, vp, u32),
     "gaast_eval": (C.c_int, vp, C.POINTER(vp), u32, vp, C.c_int, C.c_int),
     "gaast_eval_sum": (C.c_int, vp, C.POINTER(vp), u32, vp, vp, C.c_int, C.c_int),
     "gaast_eval_host": (C.c_int, vp, C.POINTER(vp), C.POINTER(u32), C.POINTER(C.c_int), u32, u64, u64, vp,

@@ -36,6 +36,7 @@ SOURCES = [
     "device/table_engine.cu",
     "device/dense_warp.cu",
     "device/dense_matrix.cu",
+    "device/records.cu",
     "device/runtime.cu",
     "device/host_pipeline.cu",
     "device/diag.cu",

@@ -201,6 +201,11 @@ gaast_status gaast_ctx_create(int device, void* stream, gaast_ctx** out) {
 gaast_status gaast_ctx_destroy(gaast_ctx* ctx) {
     return guard([&] {
         if (!ctx) return;
+        if (ctx->staging) {
+            DeviceGuard dg(ctx->device);
+            cudaStreamSynchronize(ctx->stream);
+            cudaFree(ctx->staging);
+        }
         if (ctx->h2d) cudaStreamDestroy(ctx->h2d);
         if (ctx->d2h) cudaStreamDestroy(ctx->d2h);
         if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -575,9 +580,10 @@ int gaast_batch_dtype(const gaast_batch* b) { return b ? b->dtype : GAAST_F64; }
 gaast_status gaast_batch_free(gaast_batch* b) {
     return guard([&] {
         if (!b) return;
-        if (b->owned && b->base) {
+        if ((b->owned && b->base) || !b->records.empty()) {
             DeviceGuard dg(b->ctx->device);
-            cudaFree(b->base);
+            if (b->owned && b->base) cudaFree(b->base);
+            for (auto& kv : b->records) cudaFree(kv.second.d_table);
         }
         delete b;
     });
@@ -633,6 +639,140 @@ gaast_status gaast_batch_zero(gaast_batch* b) {
                 cuda_check(cudaMemsetAsync(b->grade_ptr[k], 0, size_t(b->stored[k]) * b->stride * b->esize(), b->ctx->stream),
                            "batch zero");
     });
+}
+
+// ------------------------------------------------------------- records ----
+// Checks a records call and returns the batch's row map for `record_mask`, building it on the first call (null when
+// count == 0: nothing to do).
+static const gaast::RecordMap* records_prepare(const gaast_batch* b, uint64_t first, uint64_t count, uint32_t record_mask,
+                                               const char* what) {
+    if (!b) throw Error(GAAST_ERR_INVALID, std::string(what) + ": null batch");
+    if (!record_mask) throw Error(GAAST_ERR_SHAPE, std::string(what) + ": empty record mask (records of no component)");
+    if (record_mask & ~((2u << b->n) - 1)) throw Error(GAAST_ERR_SHAPE, std::string(what) + ": record mask has grades above n");
+    if (b->mask & ~record_mask) throw Error(GAAST_ERR_SHAPE, std::string(what) + ": the record mask lacks a grade of the batch");
+    if (b->broadcast && (first != 0 || count != 1))
+        throw Error(GAAST_ERR_SHAPE, std::string(what) + ": a broadcast batch holds one element: first = 0, count = 1");
+    if (first > b->len || count > b->len - first)
+        throw Error(GAAST_ERR_SHAPE, std::string(what) + ": first + count exceeds the batch length");
+    if (!count) return nullptr;
+    auto it = b->records.find(record_mask);
+    if (it != b->records.end()) return &it->second;
+    // stored rows in record-component order: grades ascending, within a grade the stored components ascending
+    std::vector<gaast::RecordRow> rows;
+    const size_t es = b->esize();
+    uint32_t off = 0;
+    for (uint32_t k = 0; k <= b->n; ++k) {
+        if (!(record_mask >> k & 1)) continue;
+        const uint32_t full = uint32_t(gaast::binomial(b->n, k));
+        if (b->mask >> k & 1) {
+            const std::vector<uint64_t>& present = b->present[k];
+            uint32_t rank = 0;
+            for (uint32_t c = 0; c < full; ++c) {
+                if (!present.empty() && !(present[c / 64] >> (c % 64) & 1)) continue;
+                const char* row = reinterpret_cast<const char*>(b->grade_ptr[k]) + size_t(rank++) * b->stride * es;
+                rows.push_back({reinterpret_cast<unsigned long long>(row), off + c, 0});
+            }
+        }
+        off += full;
+    }
+    gaast::RecordMap m;
+    gaast::records_shape(m, int(off), es, b->ctx->sm_count);
+    m.n_rows = rows.size();
+    std::vector<uint32_t> chunk_row(size_t(m.n_chunks) + 1);
+    for (int q = 0; q <= m.n_chunks; ++q)
+        chunk_row[size_t(q)] = uint32_t(std::lower_bound(rows.begin(), rows.end(), uint32_t(q) * uint32_t(m.Kc),
+                                                         [](const gaast::RecordRow& r, uint32_t c) { return r.comp < c; }) -
+                                        rows.begin());
+    const size_t row_bytes = rows.size() * sizeof(gaast::RecordRow), bytes = row_bytes + chunk_row.size() * sizeof(uint32_t);
+    cuda_check(cudaMalloc(&m.d_table, bytes), "cudaMalloc(record row map)");
+    cudaError_t e = cudaMemcpyAsync(m.d_table, rows.data(), row_bytes, cudaMemcpyHostToDevice, b->ctx->stream);
+    if (e == cudaSuccess)
+        e = cudaMemcpyAsync(static_cast<char*>(m.d_table) + row_bytes, chunk_row.data(), chunk_row.size() * sizeof(uint32_t),
+                            cudaMemcpyHostToDevice, b->ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(b->ctx->stream);  // (the host vectors go out of scope)
+    if (e != cudaSuccess) {
+        cudaFree(m.d_table);
+        cuda_check(e, "upload record row map");
+    }
+    return &b->records.emplace(record_mask, m).first->second;
+}
+
+// Device entry points: `records` must be device memory the kernel can address, aligned to the scalar type.
+static void records_device(const gaast_batch* b, uint64_t first, uint64_t count, void* records, uint32_t record_mask,
+                           bool unpack) {
+    const char* what = unpack ? "unpack_records" : "pack_records";
+    if (!b) throw Error(GAAST_ERR_INVALID, std::string(what) + ": null batch");
+    DeviceGuard dg(b->ctx->device);
+    const gaast::RecordMap* m = records_prepare(b, first, count, record_mask, what);
+    if (!m) return;
+    if (!records) throw Error(GAAST_ERR_INVALID, std::string(what) + ": null records pointer");
+    if (reinterpret_cast<uintptr_t>(records) % b->esize())
+        throw Error(GAAST_ERR_INVALID, std::string(what) + ": records pointer not aligned to the scalar type");
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, records) != cudaSuccess) {
+        cudaGetLastError();
+        throw Error(GAAST_ERR_INVALID, std::string(what) + ": records pointer is not known to CUDA");
+    }
+    const bool ok = attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == b->ctx->device);
+    if (!ok)
+        throw Error(GAAST_ERR_INVALID, std::string(what) + ": records pointer is not device memory of the batch's device "
+                                                           "(host records go through gaast_batch_upload_records / _download_records)");
+    cuda_check(gaast::records_launch(*m, unpack, b->esize(), records, (long long)first, (long long)count, b->ctx->stream),
+               unpack ? "launch gaast_records_unpack" : "launch gaast_records_pack");
+    b->ctx->launches++;
+}
+
+// Host entry points: chunks of GAAST_HOST_CHUNK_MIB through the ctx's staging buffer, all on the ctx stream (stream
+// order makes the reuse of the one buffer safe): copy, then pack -- or unpack, then copy.
+static void records_host(const gaast_batch* b, uint64_t first, uint64_t count, void* host, uint32_t record_mask, bool download) {
+    const char* what = download ? "download_records" : "upload_records";
+    if (!b) throw Error(GAAST_ERR_INVALID, std::string(what) + ": null batch");
+    gaast_ctx* ctx = b->ctx;
+    DeviceGuard dg(ctx->device);
+    const gaast::RecordMap* m = records_prepare(b, first, count, record_mask, what);
+    if (!m) return;
+    if (!host) throw Error(GAAST_ERR_INVALID, std::string(what) + ": null host pointer");
+    const size_t rec_bytes = size_t(m->K) * b->esize();
+    const size_t want = std::max(size_t(gaast::tuning().host_chunk_mib) << 20, rec_bytes);
+    if (ctx->staging_bytes != want) {
+        if (ctx->staging) {
+            cuda_check(cudaStreamSynchronize(ctx->stream), "staging buffer");
+            cudaFree(ctx->staging);
+            ctx->staging = nullptr;
+            ctx->staging_bytes = 0;
+        }
+        cuda_check(cudaMalloc(&ctx->staging, want), "cudaMalloc(record staging buffer)");
+        ctx->staging_bytes = want;
+    }
+    const uint64_t chunk = ctx->staging_bytes / rec_bytes;
+    char* h = static_cast<char*>(host);
+    for (uint64_t off = 0; off < count; off += chunk) {
+        const uint64_t n = std::min(chunk, count - off);
+        char* hp = h + off * rec_bytes;
+        if (!download)
+            cuda_check(cudaMemcpyAsync(ctx->staging, hp, n * rec_bytes, cudaMemcpyHostToDevice, ctx->stream), "records H2D");
+        cuda_check(gaast::records_launch(*m, download, b->esize(), ctx->staging, (long long)(first + off), (long long)n, ctx->stream),
+                   download ? "launch gaast_records_unpack" : "launch gaast_records_pack");
+        ctx->launches++;
+        if (download)
+            cuda_check(cudaMemcpyAsync(hp, ctx->staging, n * rec_bytes, cudaMemcpyDeviceToHost, ctx->stream), "records D2H");
+    }
+}
+
+gaast_status gaast_batch_pack_records(gaast_batch* b, uint64_t first, uint64_t count, const void* records, uint32_t record_mask) {
+    return guard([&] { records_device(b, first, count, const_cast<void*>(records), record_mask, false); });
+}
+gaast_status gaast_batch_unpack_records(const gaast_batch* b, uint64_t first, uint64_t count, void* records,
+                                        uint32_t record_mask) {
+    return guard([&] { records_device(b, first, count, records, record_mask, true); });
+}
+gaast_status gaast_batch_upload_records(gaast_batch* b, uint64_t first, uint64_t count, const void* host_records,
+                                        uint32_t record_mask) {
+    return guard([&] { records_host(b, first, count, const_cast<void*>(host_records), record_mask, false); });
+}
+gaast_status gaast_batch_download_records(const gaast_batch* b, uint64_t first, uint64_t count, void* host_records,
+                                          uint32_t record_mask) {
+    return guard([&] { records_host(b, first, count, host_records, record_mask, true); });
 }
 
 // ---------------------------------------------------------------- eval ----

@@ -181,6 +181,25 @@ cudaError_t dense_matrix_launch(const DenseWarpHost& prog, const DenseWarpStep& 
 struct HostPipe;
 void host_pipe_destroy(HostPipe* p);
 
+// records.cu: element-major records <-> the batch's rows.  A batch keeps one RecordMap per record mask it has
+// been packed from or unpacked to: built on the first call for that mask, so that later calls only launch.
+struct RecordRow {
+    unsigned long long ptr;  // device address of the stored row (batch column 0)
+    uint32_t comp;           // its component in the record
+    uint32_t pad;
+};
+struct RecordMap {
+    void* d_table = nullptr;  // RecordRow[n_rows], then uint32_t chunk_row[n_chunks + 1]
+    size_t n_rows = 0;
+    int K = 0, Kc = 0, E = 0, pitch = 0, n_chunks = 0, max_grid = 1;
+    size_t smem = 0;
+    int tile_scalars = 0, rows_bytes = 0, unpack_max_grid = 1;  // shared memory: the chunk's rows, then the tile (two: unpack)
+    size_t unpack_smem = 0;
+};
+void records_shape(RecordMap& m, int K, size_t es, int sm_count);
+cudaError_t records_launch(const RecordMap& m, bool unpack, size_t es, void* records, long long first, long long count,
+                           cudaStream_t stream);
+
 }  // namespace gaast
 
 struct gaast_ctx {
@@ -188,6 +207,8 @@ struct gaast_ctx {
     cudaStream_t stream = nullptr;
     bool own_stream = false;
     cudaStream_t h2d = nullptr, d2h = nullptr;  // lazily created for gaast_eval_host
+    void* staging = nullptr;  // gaast_batch_upload_records / _download_records: one chunk of records
+    size_t staging_bytes = 0;
     uint64_t launches = 0;
     int sm_count = 0;
     int smem_optin = 0;
@@ -209,6 +230,7 @@ struct gaast_batch {
     std::vector<uint64_t> present[GAAST_MAX_DIM + 1];
     uint32_t stored[GAAST_MAX_DIM + 1] = {};  // rows stored per grade
     bool sparse = false;
+    mutable std::map<uint32_t, gaast::RecordMap> records;  // by record mask (gaast_batch_pack_records / _unpack_records)
 };
 
 struct gaast_plan {

@@ -177,6 +177,52 @@ class DeviceBatch:
         ctx.sync()
         return b
 
+    @staticmethod
+    def from_records(ctx: Ctx, n: int, grades: Iterable[int], records, record_grades: Optional[Iterable[int]] = None,
+                     broadcast: bool = False, dtype: int = L.F64) -> "DeviceBatch":
+        """A batch of `grades` from element-major records (len, K_rec): one multivector per row, the components of
+        `record_grades` (default: `grades`) in slot order.  A numpy array goes through the host path, a contiguous
+        CUDA torch tensor through the device path; either must already have the batch's scalar type."""
+        grades = list(grades)
+        b = DeviceBatch.alloc(ctx, n, grades, int(records.shape[0]), broadcast, dtype)
+        b.pack_records(records, 0, grades if record_grades is None else record_grades)
+        return b
+
+    def _record_mask(self, records, record_grades) -> int:
+        mask = grade_mask(self.grade_set() if record_grades is None else record_grades)
+        width = sum(comb(self.n, k) for k in grades_of(mask))
+        assert records.ndim == 2 and records.shape[1] == width, f"records must be (count, {width})"
+        assert str(records.dtype).endswith("float32" if self.dtype == L.F32 else "float64"), "records have another dtype"
+        return mask
+
+    def pack_records(self, records, first: int = 0, record_grades: Optional[Iterable[int]] = None):
+        """Batch columns [first, first + len(records)) from records (gaast_batch_upload_records for a numpy array,
+        which returns when the copy is done; gaast_batch_pack_records, stream-ordered, for a CUDA tensor)."""
+        mask = self._record_mask(records, record_grades)
+        if isinstance(records, np.ndarray):
+            records = np.ascontiguousarray(records)
+            L.check(L.lib.gaast_batch_upload_records(self._h, int(first), records.shape[0], records.ctypes.data_as(L.vp), mask))
+            self.ctx.sync()  # `records` may be a temporary
+        else:
+            assert records.is_cuda and records.is_contiguous(), "device records must be a contiguous CUDA tensor"
+            L.check(L.lib.gaast_batch_pack_records(self._h, int(first), int(records.shape[0]), L.vp(records.data_ptr()), mask))
+
+    def to_records(self, record_grades: Optional[Iterable[int]] = None, out=None):
+        """The whole batch as records (length, K_rec) of `record_grades` (default: the batch's grades); components
+        the batch does not store are +0.  Returns a numpy array, or fills the contiguous CUDA tensor `out`
+        (stream-ordered) and returns it."""
+        if out is None:
+            width = sum(comb(self.n, k) for k in (self.grade_set() if record_grades is None else record_grades))
+            arr = np.empty((self.length, width), dtype=_np_dtype(self.dtype))
+            mask = self._record_mask(arr, record_grades)
+            L.check(L.lib.gaast_batch_download_records(self._h, 0, self.length, arr.ctypes.data_as(L.vp), mask))
+            self.ctx.sync()
+            return arr
+        mask = self._record_mask(out, record_grades)
+        assert out.is_cuda and out.is_contiguous() and out.shape[0] == self.length
+        L.check(L.lib.gaast_batch_unpack_records(self._h, 0, self.length, L.vp(out.data_ptr()), mask))
+        return out
+
     def stored_rows(self, k: int) -> int:
         return L.lib.gaast_batch_stored_rows(self._h, k)
 

@@ -285,6 +285,34 @@ gaast_status gaast_batch_download_f32(const gaast_batch* b, uint32_t grade, floa
 /* GradedDataMut::init_null_mv: zero every grade. */
 gaast_status gaast_batch_zero(gaast_batch* b);
 
+/* Element-major records: one multivector stored contiguously, as a GradedData or a Vec<[f64; K]> holds it.  A record
+ * of `record_mask` is the components of its grades, grades ascending and components in the algebra's order within a
+ * grade (the batch's slot order for that mask), K = sum over its grades of C(n,k) scalars of the batch's dtype.
+ * Records are packed without gaps: record j (batch column first + j) starts at scalar j * K.  The record scalar type
+ * is the batch's, so the pointers are untyped; scalars are copied bit for bit (-0.0, subnormals, NaN payloads).
+ * GAAST_ERR_SHAPE when record_mask is empty or lacks a grade of the batch, when first + count > len, or when a
+ * broadcast batch is given anything but first = 0, count = 1; GAAST_ERR_INVALID for a null batch, or a null pointer with count > 0.
+ * count == 0 returns GAAST_OK and launches nothing.  The first call for a given record_mask builds the batch's
+ * row map for it (a device table freed by gaast_batch_free); every later call only enqueues its kernel(s) on the
+ * ctx stream and can be captured in a CUDA graph. */
+/* Device records -> batch columns [first, first + count).  `records` is device memory of the batch's device (or
+ * managed memory) holding `count` records of record_mask, which must include every grade of the batch; another
+ * pointer is GAAST_ERR_INVALID, checked before any launch.  Components the batch does not store (other grades, absent
+ * components of a sparse grade) are ignored.  One kernel launch on the ctx stream. */
+gaast_status gaast_batch_pack_records(gaast_batch* b, uint64_t first, uint64_t count, const void* records,
+                                      uint32_t record_mask);
+/* Batch columns [first, first + count) -> `count` device records of record_mask.  EVERY component of every record is
+ * written: the batch's value where it stores one, +0 elsewhere (the element as a multivector of record_mask). */
+gaast_status gaast_batch_unpack_records(const gaast_batch* b, uint64_t first, uint64_t count, void* records,
+                                        uint32_t record_mask);
+/* The same from / to host memory (pageable or page-locked), through a device staging buffer owned by the ctx, in
+ * chunks of GAAST_HOST_CHUNK_MIB: per chunk a copy and a kernel launch.  Stream-ordered like gaast_batch_upload /
+ * _download: synchronise the ctx before reading downloaded records or reusing uploaded ones in page-locked memory. */
+gaast_status gaast_batch_upload_records(gaast_batch* b, uint64_t first, uint64_t count, const void* host_records,
+                                        uint32_t record_mask);
+gaast_status gaast_batch_download_records(const gaast_batch* b, uint64_t first, uint64_t count, void* host_records,
+                                          uint32_t record_mask);
+
 /* eval: out[i] = expr(inputs[0][i], inputs[1][i], ...) for i in [0, len).
  * `inputs` has plan.n_slots entries; `out` must carry exactly the plan's root
  * grade set (SURVEY.md Q3).  Stream-ordered, asynchronous. */

@@ -158,6 +158,10 @@ extern "C" {
     pub fn gaast_batch_upload_f32(b: *mut gaast_batch, grade: u32, host: *const f32, host_stride: u64) -> c_int;
     pub fn gaast_batch_download_f32(b: *const gaast_batch, grade: u32, host: *mut f32, host_stride: u64) -> c_int;
     pub fn gaast_batch_zero(b: *mut gaast_batch) -> c_int;
+    pub fn gaast_batch_pack_records(b: *mut gaast_batch, first: u64, count: u64, records: *const c_void, record_mask: u32) -> c_int;
+    pub fn gaast_batch_unpack_records(b: *const gaast_batch, first: u64, count: u64, records: *mut c_void, record_mask: u32) -> c_int;
+    pub fn gaast_batch_upload_records(b: *mut gaast_batch, first: u64, count: u64, host_records: *const c_void, record_mask: u32) -> c_int;
+    pub fn gaast_batch_download_records(b: *const gaast_batch, first: u64, count: u64, host_records: *mut c_void, record_mask: u32) -> c_int;
 
     pub fn gaast_eval(plan: *mut gaast_plan, inputs: *const *mut gaast_batch, n_inputs: u32, out: *mut gaast_batch, engine: c_int, arith: c_int) -> c_int;
     pub fn gaast_eval_sum(plan: *mut gaast_plan, inputs: *const *mut gaast_batch, n_inputs: u32, out: *mut gaast_batch, dev_sum: *mut f64, engine: c_int, arith: c_int) -> c_int;
