@@ -103,6 +103,7 @@ PROTOTYPES = {
     "gaast_ctx_stream": (vp, vp),
     "gaast_ctx_launch_count": (u64, vp),
     "gaast_plan_create": (C.c_int, vp, C.POINTER(PlanDesc), C.POINTER(vp)),
+    "gaast_plan_create_projected": (C.c_int, vp, C.POINTER(PlanDesc), C.POINTER(C.POINTER(u64)), C.POINTER(vp)),
     "gaast_plan_destroy": (C.c_int, vp),
     "gaast_plan_cost": (C.c_int, vp, u64, C.POINTER(u64), C.POINTER(u64)),
     "gaast_plan_root_mask": (u32, vp),

@@ -100,6 +100,11 @@ struct Gen {
     Gen(const DevicePlanHost& hh, const CodegenOptions& o)
         : h(hh), opt(o), strict(o.arith == GAAST_ARITH_STRICT), f32(o.f32), S(o.f32 ? "float" : "double"), esize(o.f32 ? 4 : 8) {}
 
+    // A projected plan stores root column `col` only when root_row[col] >= 0.  With `prune`, root liveness starts from
+    // those columns alone (set after the lowering passes, which match patterns on the whole root buffer).
+    bool prune = false;
+    bool stored(size_t col) const { return h.root_row[col] >= 0; }
+
     int add(const Node& n) {
         nodes.push_back(n);
         return int(nodes.size()) - 1;
@@ -682,7 +687,8 @@ struct Gen {
 
     void mark_live() {
         std::vector<int> stack;
-        for (Ref r : buf[0]) stack.push_back(r.id);
+        for (size_t col = 0; col < buf[0].size(); ++col)
+            if (!prune || stored(col)) stack.push_back(buf[0][col].id);
         while (!stack.empty()) {
             const int id = stack.back();
             stack.pop_back();
@@ -725,7 +731,8 @@ struct Gen {
                 want(n.a);
             }
         }
-        for (Ref r : buf[0]) want(r);
+        for (size_t col = 0; col < buf[0].size(); ++col)
+            if (stored(col)) want(buf[0][col]);
     }
 
     void compute_blades() {
@@ -961,8 +968,9 @@ struct Gen {
     // exists, so that finished outputs do not occupy registers.
     struct RootSlot {
         size_t stream;
-        uint32_t row, col;
+        uint32_t row, col;  // row: among the grade's stored rows; col: root column
         bool neg;
+        uint32_t sum_col;   // batch-sum column (rank among the stored root components)
     };
     std::multimap<int, RootSlot> root_of;  // node id -> root slots holding it
     std::vector<char> root_done;
@@ -975,7 +983,7 @@ struct Gen {
             line("d_store(s" + std::to_string(rs.stream) + " + " + std::to_string(rs.row) + " * r" +
                  std::to_string(rs.stream) + " + e, " + val + ");");
         if (sum_in_smem)
-            line(guard + "sums[" + std::to_string(rs.col) + " * GAAST_THREADS + tid] += d_hsum(" + val + ");");
+            line(guard + "sums[" + std::to_string(rs.sum_col) + " * GAAST_THREADS + tid] += d_hsum(" + val + ");");
         if (sum_in_tmem) {
             // Accumulators are numbered in emission order (column pair 2k for the k-th finished
             // component).  The first `sum_stash` components only park their value in a second
@@ -983,15 +991,15 @@ struct Gen {
             // absorb the whole stash at the end of the tile, 16 components per
             // tcgen05.ld/st.  Components beyond the stash capacity are added one by one.
             const size_t k = sum_order.size();
-            sum_order.push_back(rs.col);
+            sum_order.push_back(rs.sum_col);
             if (k < sum_stash)
-                line("tm_put(tb + " + std::to_string(2 * root_done.size() + 2 * k) + "u, d_hsum(" + val + "));");
+                line("tm_put(tb + " + std::to_string(2 * h.stored_cols + 2 * k) + "u, d_hsum(" + val + "));");
             else  // warp-collective: idle lanes add zero
                 line("tm_add(tb + " + std::to_string(2 * k) + "u, active ? d_hsum(" + val + ") : 0.0);");
         }
     }
     size_t sum_stash = 0;             // components whose per-tile value is parked in tensor memory
-    std::vector<uint32_t> sum_order;  // root columns in the order their sums are updated
+    std::vector<uint32_t> sum_order;  // batch-sum columns in the order their sums are updated
     void store_if_root(int id) {
         if (in_prologue) return;
         auto range = root_of.equal_range(id);
@@ -1194,6 +1202,9 @@ struct Gen {
         for (size_t b = 0; b < B; ++b) any_right_neg |= bool(d.right_neg[b]);
         if (d.unit_sigma) plan_matrep(d, coeff);
         if (any_right_neg && !d.mr.ok) return false;  // only the matrix path takes per-blade signs
+        // a projected root: the rolled product stores whole cosets, and its 4^n FMAs are never fewer than the terms
+        // of the selected components -- only the matrix path (fewer FMAs than the full table) is kept
+        if (h.projected && !d.mr.ok) return false;
         dense = d;
         return true;
     }
@@ -1381,9 +1392,9 @@ struct Gen {
     void emit_op_dense_matrep(int op) {
         const Dense& d = dense;
         const MatRep& m = d.mr;
-        std::vector<std::pair<size_t, uint32_t>> col_at;
+        std::vector<std::pair<size_t, uint32_t>> col_at;  // root column -> (stream, stored row)
         for (size_t si = h.n_in_streams; si < h.streams.size(); ++si)
-            for (uint32_t r = 0; r < h.streams[si].rows; ++r) col_at.push_back({si, r});
+            for (uint32_t r = 0; r < h.streams[si].rows; ++r) col_at.push_back({si, uint32_t(h.root_row[col_at.size()])});
         const int g = m.group, ja = g == 0 ? 1 : 0, jb = g == 2 ? 1 : 2;  // the group factor and the two others (ja < jb)
         const int st[3] = {1, 4, 16};
         auto T = [&](int kg, int ka, int kb) { return kg * st[g] + ka * st[ja] + kb * st[jb]; };
@@ -1508,7 +1519,9 @@ struct Gen {
             for (int ka = 0; ka < 4; ++ka)
                 for (int kb = 0; kb < 4; ++kb) {
                     const int tau = T(og, ka, kb);
-                    const auto at = col_at[size_t(d.out_col[size_t(m.tau_blade[tau])])];
+                    const size_t oc = size_t(d.out_col[size_t(m.tau_blade[tau])]);
+                    if (!stored(oc)) continue;  // (projected away: computed, never stored)
+                    const auto at = col_at[oc];
                     const double f = scale * m.tau_sign[tau] * cout[ka][kb].sign;
                     const std::string v = f == 1.0 ? cout[ka][kb].text : "d_mul(U(" + lit(f) + "), " + cout[ka][kb].text + ")";
                     if (opt.store_out)
@@ -1954,7 +1967,7 @@ __device__ __forceinline__ float d_logf(float a, float q) { return (float)s_logf
 
 }  // namespace
 
-CodegenResult generate_kernel(const DevicePlanHost& h, const CodegenOptions& opt) {
+static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt, bool prune) {
     Gen g(h, opt);
     g.build();
     g.mark_live();
@@ -2001,6 +2014,12 @@ CodegenResult generate_kernel(const DevicePlanHost& h, const CodegenOptions& opt
             throw Error(GAAST_ERR_JIT, "plan too large for the specialised engine (" + std::to_string(live_terms) +
                                            " live terms): use the table engine");
     }
+    if (prune) {
+        g.prune = true;
+        for (Node& n : g.nodes) n.live = false;
+        g.mark_live();
+    }
+    if (h.projected) notes << "projection(" << h.stored_cols << "/" << h.buf_cols[0] << (prune ? ",pruned" : ",whole") << ") ";
     g.mark_exports();
     g.compute_blades();
 
@@ -2008,7 +2027,7 @@ CodegenResult generate_kernel(const DevicePlanHost& h, const CodegenOptions& opt
     size_t live_loads = 0;
     for (const Node& n : g.nodes)
         if (n.live && n.k == N_LOAD && !n.uniform) ++live_loads;
-    const size_t root_cols = h.buf_cols[0];
+    const size_t root_cols = h.stored_cols;  // batch-sum columns
     // (an f32 value takes one register instead of two: the budgets below nearly double)
     const size_t kAccBudget = opt.f32 ? 128 : 72;  // values a thread can keep as accumulators next to its operands
     g.op_policy.assign(h.ops.size() + 1, P_TABLE);
@@ -2284,7 +2303,8 @@ CodegenResult generate_kernel(const DevicePlanHost& h, const CodegenOptions& opt
             if (!n.live || n.uniform) continue;
             used[n.a.id] = used[n.b.id] = used[n.c.id] = 1;
         }
-        for (Ref r : g.buf[0]) used[r.id] = 1;
+        for (size_t col = 0; col < g.buf[0].size(); ++col)
+            if (g.stored(col)) used[g.buf[0][col].id] = 1;
         // a handful of shared values live in registers for the whole kernel; a large table of
         // them (a wide linear map) is read at its point of use instead (uniform, L1-resident)
         size_t n_shared = 0;
@@ -2307,12 +2327,13 @@ CodegenResult generate_kernel(const DevicePlanHost& h, const CodegenOptions& opt
     }
     // root components, in slot order
     {
-        std::vector<Gen::RootSlot> slots;
+        std::vector<Gen::RootSlot> slots;  // the stored ones (a projected plan: the selected components)
         uint32_t col = 0;
         for (size_t si = h.n_in_streams; si < h.streams.size(); ++si)
             for (uint32_t r = 0; r < h.streams[si].rows; ++r, ++col)
-                slots.push_back(Gen::RootSlot{si, r, col, g.buf[0][col].neg});
-        g.root_done.assign(slots.size(), 0);
+                if (g.stored(col))
+                    slots.push_back(Gen::RootSlot{si, uint32_t(h.root_row[col]), col, g.buf[0][col].neg, uint32_t(h.root_sum_col[col])});
+        g.root_done.assign(h.buf_cols[0], 0);
         g.root_of.clear();
         // one-tile blocks with TMA staging: the parked rows are already on their way to shared
         // memory (bulk copies issued by thread 0 at kernel start); otherwise LDG + STS here
@@ -2598,6 +2619,20 @@ CodegenResult generate_kernel(const DevicePlanHost& h, const CodegenOptions& opt
     res.source = src.str();
     res.notes = notes.str();
     return res;
+}
+
+CodegenResult generate_kernel(const DevicePlanHost& h, const CodegenOptions& opt) {
+    if (!h.projected) return generate(h, opt, false);
+    // A projected plan: root liveness from the selected components drops every term that feeds only the others.  A
+    // matrix-representation product needs all of its outputs, so it only survives in the kernel that keeps the whole
+    // root live (and stores the selected components): that kernel is taken when it executes fewer FMAs.
+    CodegenResult pruned = generate(h, opt, true);
+    try {
+        CodegenResult whole = generate(h, opt, false);
+        if (whole.fma_per_elem < pruned.fma_per_elem) return whole;
+    } catch (const Error&) {
+    }
+    return pruned;
 }
 
 }  // namespace gaast

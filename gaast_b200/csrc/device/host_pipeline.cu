@@ -101,6 +101,9 @@ static gaast_status eval_host_impl(gaast_plan* plan, const void* const* host_in_
         if (!plan || !plan->ctx) throw Error(GAAST_ERR_INVALID, "eval_host: null or offline plan");
         gaast_ctx* ctx = plan->ctx;
         const auto& h = plan->h;
+        if (h.projected)
+            throw Error(GAAST_ERR_UNSUPPORTED, "eval_host: a projected plan (gaast_plan_create_projected) writes a sparse "
+                                               "output batch: evaluate it with gaast_eval on device batches");
         if (n_inputs != h.n_slots) throw Error(GAAST_ERR_SHAPE, "eval_host: wrong number of inputs");
         if ((n_inputs && (!host_in || !in_masks || !in_broadcast)) || !host_out)
             throw Error(GAAST_ERR_INVALID, "eval_host: null argument");

@@ -92,7 +92,16 @@ void bind_streams(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_input
         if (out->mask != h.buffer_masks[0])
             throw Error(GAAST_ERR_SHAPE, "eval: output batch must carry exactly the root grade set");
         if (out->broadcast) throw Error(GAAST_ERR_SHAPE, "eval: output batch cannot be a broadcast operand");
-        if (out->sparse) throw Error(GAAST_ERR_SHAPE, "eval: the output batch must be dense (sparse storage is for inputs)");
+        if (!h.projected) {
+            if (out->sparse)
+                throw Error(GAAST_ERR_SHAPE, "eval: the output batch must be dense (sparse storage is for inputs and for "
+                                             "the results of projected plans)");
+        } else {
+            for (uint32_t i = h.n_in_streams; i < h.streams.size(); ++i)
+                if (out->present[h.streams[i].grade] != h.root_present[i - h.n_in_streams])
+                    throw Error(GAAST_ERR_SHAPE, "eval: the output batch must store exactly the components the projected "
+                                                 "plan keeps (grade " + std::to_string(h.streams[i].grade) + " differs)");
+        }
         n = (long long)out->len;
     } else if (need_out) {
         throw Error(GAAST_ERR_INVALID, "eval: null output batch");
@@ -140,7 +149,7 @@ void bind_streams(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_input
     // an output array overlapping an input array would be read after it was overwritten
     for (size_t o = h.n_in_streams; o < h.streams.size() && out; ++o) {
         const char* ob = reinterpret_cast<const char*>(a.sptr[o]);
-        const char* oe = ob + size_t(h.streams[o].rows) * size_t(a.srow[o]) * esize;
+        const char* oe = ob + size_t(h.stored_rows(o)) * size_t(a.srow[o]) * esize;
         for (size_t i = 0; i < h.n_in_streams; ++i) {
             const char* ib = reinterpret_cast<const char*>(a.sptr[i]);
             const gaast_batch* ibatch = inputs[h.streams[i].slot];
@@ -256,14 +265,15 @@ void* gaast_ctx_stream(gaast_ctx* ctx) { return ctx ? ctx->stream : nullptr; }
 uint64_t gaast_ctx_launch_count(gaast_ctx* ctx) { return ctx ? ctx->launches : 0; }
 
 // ---------------------------------------------------------------- plan ----
-gaast_status gaast_plan_create(gaast_ctx* ctx, const gaast_plan_desc* desc, gaast_plan** out) {
+static gaast_status plan_create(gaast_ctx* ctx, const gaast_plan_desc* desc, const uint64_t* const* root_present,
+                                gaast_plan** out) {
     return guard([&] {
         if (!out) throw Error(GAAST_ERR_INVALID, "null output pointer");
         *out = nullptr;
         if (!desc) throw Error(GAAST_ERR_INVALID, "null plan description");
         auto plan = std::make_unique<gaast_plan>();
         plan->ctx = ctx;
-        plan->h.build(*desc);
+        plan->h.build(*desc, root_present);
         if (ctx) {
             DeviceGuard dg(ctx->device);
             upload(plan->d_micro, plan->h.micro, ctx->stream);
@@ -273,6 +283,20 @@ gaast_status gaast_plan_create(gaast_ctx* ctx, const gaast_plan_desc* desc, gaas
         }
         *out = plan.release();
     });
+}
+
+gaast_status gaast_plan_create(gaast_ctx* ctx, const gaast_plan_desc* desc, gaast_plan** out) {
+    return plan_create(ctx, desc, nullptr, out);
+}
+
+gaast_status gaast_plan_create_projected(gaast_ctx* ctx, const gaast_plan_desc* desc, const uint64_t* const* root_present,
+                                         gaast_plan** out) {
+    if (out) *out = nullptr;
+    if (!root_present) {
+        gaast::set_last_error("plan_create_projected: null root bitmap array");
+        return GAAST_ERR_INVALID;
+    }
+    return plan_create(ctx, desc, root_present, out);
 }
 
 gaast_status gaast_plan_destroy(gaast_plan* plan) {
@@ -311,9 +335,10 @@ gaast_status gaast_plan_cost(const gaast_plan* plan, uint64_t broadcast_slots, u
         if (!plan) throw Error(GAAST_ERR_INVALID, "null plan");
         const auto& h = plan->h;
         uint64_t doubles = 0;
-        for (const auto& st : h.streams) {
+        for (size_t i = 0; i < h.streams.size(); ++i) {
+            const auto& st = h.streams[i];
             if (st.slot != 0xFFFFFFFFu && (broadcast_slots >> st.slot & 1)) continue;
-            doubles += st.rows;
+            doubles += h.stored_rows(i);  // (a projected root: its stored components only)
         }
         if (bytes_per_elem) *bytes_per_elem = 8 * doubles;
         if (flops_per_elem) *flops_per_elem = 2 * h.total_terms;
@@ -425,7 +450,7 @@ gaast_status gaast_plan_precompile_typed(gaast_plan* plan, uint64_t broadcast_sl
         } catch (const Error&) {
             // too large / too wide to specialise: a full high-dimensional product gets its dense-warp kernel instead
             gaast::DenseWarpHost dw;
-            if (opt.f32 || opt.with_sum || arith != GAAST_ARITH_FMA || !gaast::dense_warp_analyse(plan->h, &dw)) throw;
+            if (opt.f32 || opt.with_sum || arith != GAAST_ARITH_FMA || plan->h.projected || !gaast::dense_warp_analyse(plan->h, &dw)) throw;
             gaast_ctx fake;  // offline: the launch shape of a B200 (227 KB of shared memory per block, 148 SMs)
             fake.sm_count = 148;
             fake.smem_optin = 232448;
@@ -824,7 +849,7 @@ static void eval_impl(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_i
                                            "generated for the sparsity pattern): use GAAST_ENGINE_AUTO or GAAST_ENGINE_SPECIALIZED");
     const bool f32 = dtype == GAAST_F32;
     const gaast::DevicePlanHost& h = plan->h;
-    const int sum_cols = int(h.buf_cols[0]);
+    const int sum_cols = int(h.stored_cols);  // one column per stored root component
     a.n_sum_cols = with_sum ? sum_cols : 0;
     if (n == 0) {
         if (with_sum) cuda_check(cudaMemsetAsync(dev_sum, 0, sum_cols * sizeof(double), ctx->stream), "zero sum");
@@ -902,6 +927,9 @@ static void eval_impl(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_i
         return true;
     };
     bool use_dense_warp = false;
+    if (engine == GAAST_ENGINE_DENSE_WARP && h.projected)
+        throw Error(GAAST_ERR_UNSUPPORTED, "dense-warp engine: a projected plan is evaluated by the specialised or the "
+                                           "table engine");
     if (engine == GAAST_ENGINE_DENSE_WARP) {
         if (!dense_warp_ready())
             throw Error(GAAST_ERR_UNSUPPORTED,
@@ -974,7 +1002,7 @@ static void eval_impl(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_i
         // the table engine at n = 7, 8 -- worth it while the plan keeps at least 1/8 of the pairs; at n = 9, 10 the
         // table engine's workspace is in global memory (0.09 TFLOP/s): 1/64.  exp/rotor_square.py, exp/big_products.py)
         const double min_density = h.n <= 8 ? 1.0 / 8.0 : 1.0 / 64.0;
-        if (!jk && engine == GAAST_ENGINE_AUTO && dense_warp_ready() &&
+        if (!jk && engine == GAAST_ENGINE_AUTO && !h.projected && dense_warp_ready() &&
             double(h.total_terms) >= min_density * double(plan->dense_warp.steps.size()) * std::pow(4.0, double(h.n)))
             use_dense_warp = true;
     } else if (engine != GAAST_ENGINE_TABLE && engine != GAAST_ENGINE_AUTO) {

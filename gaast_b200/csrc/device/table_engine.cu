@@ -254,7 +254,7 @@ __global__ void __launch_bounds__(256) table_engine_kernel(const __grid_constant
                         const T v = w[size_t(op.dst_col + r) * kLanes];
                         if (active && a.store_out) dst[r * rs] = v;
                         if (kSum && active) {
-                            double* sc = &sw[size_t((op.dst_col - a.root_col) + r) * kLanes];
+                            double* sc = &sw[size_t(op.pad0 + r) * kLanes];  // (pad0: the run's first batch-sum column)
                             *sc = *sc + double(v);
                         }
                     }
@@ -345,9 +345,9 @@ cudaError_t launch_s(const EvalArgs& args, const TableLaunch& shape, bool strict
 
 TableLaunch table_engine_shape(const gaast_ctx& ctx, const DevicePlanHost& h, long long n, bool with_sum, bool f32) {
     TableLaunch s;
-    const size_t cols = h.total_cols + (with_sum ? h.buf_cols[0] : 0);
+    const size_t cols = h.total_cols + (with_sum ? h.stored_cols : 0);
     // one tile = 32 elements; the sum columns are doubles in both variants
-    const size_t ws_bytes = (h.total_cols * (f32 ? sizeof(float) : sizeof(double)) + (with_sum ? h.buf_cols[0] * sizeof(double) : 0)) * kLanes;
+    const size_t ws_bytes = (h.total_cols * (f32 ? sizeof(float) : sizeof(double)) + (with_sum ? h.stored_cols * sizeof(double) : 0)) * kLanes;
     s.threads = 256;                                         // 8 warps share the tile's work
     s.global_ws = kWsOffset + ws_bytes > size_t(ctx.smem_optin);
     s.smem = s.global_ws ? kWsOffset : kWsOffset + ws_bytes;

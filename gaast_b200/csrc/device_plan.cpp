@@ -28,7 +28,15 @@ int DevicePlanHost::stream_of(uint32_t slot, uint32_t grade) const {
     return -1;
 }
 
-void DevicePlanHost::build(const gaast_plan_desc& d) {
+uint32_t DevicePlanHost::stored_rows(size_t stream) const {
+    const Stream& st = streams[stream];
+    if (st.slot != 0xFFFFFFFFu || root_present[stream - n_in_streams].empty()) return st.rows;
+    uint32_t c = 0;
+    for (uint64_t w : root_present[stream - n_in_streams]) c += uint32_t(__builtin_popcountll(w));
+    return c;
+}
+
+void DevicePlanHost::build(const gaast_plan_desc& d, const uint64_t* const* present) {
     auto bad = [](const std::string& m) { throw Error(GAAST_ERR_INVALID, "plan: " + m); };
     if (d.n > GAAST_MAX_DIM) bad("dimension above GAAST_MAX_DIM");
     if (d.n_buffers == 0 || !d.buffer_masks) bad("no buffers (buffer 0 must be the root)");
@@ -146,6 +154,32 @@ void DevicePlanHost::build(const gaast_plan_desc& d) {
         if (buffer_masks[0] >> k & 1) streams.push_back(Stream{0xFFFFFFFFu, k, gdim[k]});
     if (streams.size() > size_t(kMaxStreams)) bad("too many (input, grade) arrays for one kernel");
 
+    // projection: normalised as gaast_batch_alloc_sparse normalises a batch's bitmaps (bits past C(n,k) ignored, a
+    // grade with every bit set is dense), so that a batch allocated from the same bitmaps matches the plan
+    projected = false;
+    root_present.assign(streams.size() - n_in_streams, {});
+    root_row.assign(buf_cols[0], -1);
+    root_sum_col.assign(buf_cols[0], -1);
+    stored_cols = 0;
+    for (size_t i = n_in_streams, col = 0; i < streams.size(); ++i) {
+        const uint32_t full = streams[i].rows;
+        std::vector<uint64_t>& bits = root_present[i - n_in_streams];
+        if (present && present[i - n_in_streams]) {
+            bits.assign(present[i - n_in_streams], present[i - n_in_streams] + (full + 63) / 64);
+            if (full % 64) bits.back() &= (~0ull) >> (64 - full % 64);
+            uint32_t cnt = 0;
+            for (uint64_t w : bits) cnt += uint32_t(__builtin_popcountll(w));
+            if (cnt == full) bits.clear();
+            else projected = true;
+        }
+        for (uint32_t c = 0, row = 0; c < full; ++c, ++col)
+            if (bits.empty() || (bits[c / 64] >> (c % 64) & 1)) {
+                root_row[col] = int32_t(row++);
+                root_sum_col[col] = int32_t(stored_cols++);
+            }
+    }
+    if (present && stored_cols == 0) throw Error(GAAST_ERR_SHAPE, "plan: the projection stores no root component");
+
     micro.clear();
     chunks.clear();
     auto push = [&](uint32_t kind, uint32_t dst, uint32_t a, uint32_t b, uint32_t count, uint32_t chunk0 = 0) {
@@ -209,8 +243,19 @@ void DevicePlanHost::build(const gaast_plan_desc& d) {
             }
         }
     }
-    for (uint32_t i = n_in_streams; i < streams.size(); ++i)
-        push(MK_STORE, col_of(0, streams[i].grade), i, 0, streams[i].rows);
+    // one store per run of consecutive stored components: workspace column, stream, first stored row, count, and
+    // (pad0) the run's first batch-sum column
+    for (uint32_t i = n_in_streams; i < streams.size(); ++i) {
+        const uint32_t c0 = col_of(0, streams[i].grade) - buf_col[0];
+        for (uint32_t c = c0; c < c0 + streams[i].rows;) {
+            if (root_row[c] < 0) { ++c; continue; }
+            uint32_t e = c;
+            while (e < c0 + streams[i].rows && root_row[e] >= 0) ++e;
+            push(MK_STORE, buf_col[0] + c, i, uint32_t(root_row[c]), e - c);
+            micro.back().pad0 = uint32_t(root_sum_col[c]);
+            c = e;
+        }
+    }
 }
 
 }  // namespace gaast

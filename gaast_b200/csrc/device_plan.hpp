@@ -34,7 +34,8 @@ struct MicroOp {
     uint32_t b;        // LOAD_ADD/STORE: first row in the stream; MUL: right column base
     uint32_t count;    // rows / columns; MUL: number of chunks
     uint32_t chunk0;   // MUL: first chunk record
-    uint32_t pad0, pad1;
+    uint32_t pad0;     // STORE: first batch-sum column of the run
+    uint32_t pad1;
 };
 
 // A fixed-size record the table engine pulls into shared memory with one
@@ -69,11 +70,20 @@ struct DevicePlanHost {
     std::vector<MicroOp> micro;
     std::vector<TermChunk> chunks;
     uint64_t total_terms = 0;
+    // Projection of the root (gaast_plan_create_projected): the root components the plan stores.  `projected` is set
+    // only when some grade is partly selected; a grade with every component selected is dense (empty bitmap).
+    bool projected = false;
+    std::vector<std::vector<uint64_t>> root_present;  // per root grade, ascending: bitmap of stored components (empty = all)
+    std::vector<int32_t> root_row;      // per root column: its row in its grade's array (rank among the stored), -1 = not stored
+    std::vector<int32_t> root_sum_col;  // per root column: its batch-sum column (rank among all stored components), -1
+    uint32_t stored_cols = 0;           // stored root components: the width of the batch-sum vector
 
     uint32_t col_of(uint32_t buf, uint32_t grade) const;  // first column of `grade` inside `buf`
     int stream_of(uint32_t slot, uint32_t grade) const;
-    // Throws gaast::Error on malformed descriptions.
-    void build(const gaast_plan_desc& d);
+    uint32_t stored_rows(size_t stream) const;  // rows of a stream's array: C(n,k), or the projected count for the root
+    // Throws gaast::Error on malformed descriptions.  `root_present` (one bitmap pointer per root grade, null = the
+    // whole grade) projects the root onto the components it selects.
+    void build(const gaast_plan_desc& d, const uint64_t* const* root_present = nullptr);
 };
 
 }  // namespace gaast

@@ -140,6 +140,19 @@ class DeviceBatch:
         return b
 
     @staticmethod
+    def alloc_sparse(ctx: Ctx, n: int, components: Dict[int, Optional[Iterable[int]]], length: int,
+                     broadcast: bool = False, dtype: int = L.F64) -> "DeviceBatch":
+        """An uninitialised batch in sparse per-grade storage (gaast_batch_alloc_sparse): components[grade] = the
+        stored component indices, or None for a dense grade."""
+        grades = sorted(components)
+        bitmaps = [_bitmap(n, k, components[k]) for k in grades]
+        ptrs = (C.POINTER(L.u64) * max(1, len(grades)))(*[C.cast(b, C.POINTER(L.u64)) if b is not None else None for b in bitmaps])
+        out = L.vp()
+        L.check(L.lib.gaast_batch_alloc_sparse(ctx._h, n, grade_mask(grades), int(length), int(broadcast), int(dtype), ptrs,
+                                               C.byref(out)))
+        return DeviceBatch(out, ctx, n)
+
+    @staticmethod
     def from_host_sparse(ctx: Ctx, n: int, data: Dict[int, "tuple"], broadcast: bool = False,
                          dtype: int = L.F64) -> "DeviceBatch":
         """Sparse per-grade storage (gaast_batch_alloc_sparse): data[grade] = (stored component indices, array
@@ -279,13 +292,28 @@ class DeviceBatch:
 
 
 class Plan:
-    """gaast_plan: a lowered SpecializedAst, reusable with new inputs."""
+    """gaast_plan: a lowered SpecializedAst, reusable with new inputs.
 
-    def __init__(self, ctx: Optional[Ctx], ast: SpecializedAst):
+    `components` = {root grade: [component indices]} makes a projected plan (gaast_plan_create_projected): only those
+    components of the listed grades are stored, a grade that is not listed is kept whole, and the result is a sparse
+    output batch (`alloc_output` allocates the matching one)."""
+
+    def __init__(self, ctx: Optional[Ctx], ast: SpecializedAst, components: Optional[Dict[int, Iterable[int]]] = None):
         self.ctx = ctx
         self.ast = ast  # owns the plan description
         out = L.vp()
-        L.check(L.lib.gaast_plan_create(ctx._h if ctx else None, ast.lower(), C.byref(out)))
+        self.components = None
+        if components is None:
+            L.check(L.lib.gaast_plan_create(ctx._h if ctx else None, ast.lower(), C.byref(out)))
+        else:
+            desc = ast.lower()
+            n, grades = desc.contents.n, grades_of(desc.contents.buffer_masks[0])
+            assert set(components) <= set(grades), "components of a grade the root does not have"
+            self.components = {k: (sorted(int(i) for i in components[k]) if k in components else None) for k in grades}
+            bitmaps = [_bitmap(n, k, self.components[k]) for k in grades]
+            ptrs = (C.POINTER(L.u64) * max(1, len(grades)))(*[C.cast(b, C.POINTER(L.u64)) if b is not None else None
+                                                               for b in bitmaps])
+            L.check(L.lib.gaast_plan_create_projected(ctx._h if ctx else None, desc, ptrs, C.byref(out)))
         self._h = out
         self.n = L.lib.gaast_plan_dim(out)
 
@@ -343,6 +371,9 @@ class Plan:
         return (L.lib.gaast_plan_last_kernel(self._h) or b"").decode()
 
     def alloc_output(self, length: int, dtype: int = L.F64) -> DeviceBatch:
+        """The output batch `eval` writes: dense, or for a projected plan sparse in the plan's components."""
+        if self.components is not None:
+            return DeviceBatch.alloc_sparse(self.ctx, self.n, self.components, length, dtype=dtype)
         return DeviceBatch.alloc(self.ctx, self.n, self.root_grades(), length, dtype=dtype)
 
     def eval(self, inputs: Sequence[DeviceBatch], out: Optional[DeviceBatch] = None, engine: int = L.ENGINE_AUTO,
@@ -359,6 +390,8 @@ class Plan:
 
     def eval_sum(self, inputs: Sequence[DeviceBatch], dev_sum_ptr: int, out: Optional[DeviceBatch] = None,
                  engine: int = L.ENGINE_AUTO, arith: int = L.ARITH_FMA):
+        """Writes sum_i out[i] to `dev_sum_ptr` (device memory): one double per root component, or for a projected
+        plan one per stored component (grades ascending, stored components ascending).  `out` may be None."""
         arr = (L.vp * max(1, len(inputs)))(*[b._h for b in inputs])
         L.check(L.lib.gaast_eval_sum(self._h, arr, len(inputs), out._h if out else None, L.vp(dev_sum_ptr), engine,
                                      arith))
@@ -477,6 +510,17 @@ def pin_host(a: np.ndarray):
     """Pins an existing numpy array in place (gaast_host_register); returns a callable that unpins it."""
     L.check(L.lib.gaast_host_register(L.vp(a.ctypes.data), a.nbytes))
     return lambda: L.check(L.lib.gaast_host_unregister(L.vp(a.ctypes.data)))
+
+
+def _bitmap(n: int, k: int, idx: Optional[Iterable[int]]):
+    """gaast_batch_alloc_sparse's presence bitmap of grade k (None = the whole grade)."""
+    if idx is None:
+        return None
+    bits = (L.u64 * ((comb(n, k) + 63) // 64))()
+    for i in idx:
+        assert 0 <= int(i) < comb(n, k), f"component {i} outside grade {k}"
+        bits[int(i) // 64] |= 1 << (int(i) % 64)
+    return bits
 
 
 def _is_broadcast(b: DeviceBatch) -> bool:

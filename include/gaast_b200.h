@@ -197,10 +197,33 @@ uint64_t gaast_ctx_launch_count(gaast_ctx* ctx);
 /* plan: validates `desc` (copying everything it needs) and uploads its tables.
  * ctx may be NULL for an offline plan (kernel_source / precompile only). */
 gaast_status gaast_plan_create(gaast_ctx* ctx, const gaast_plan_desc* desc, gaast_plan** out);
+/* A projected plan: the same expression, keeping only chosen root components (a component-level counterpart of
+ * the grade projection .g(k)); the others are zero, and the result is a SPARSE output batch (gaast_batch_alloc_sparse
+ * with the same bitmaps).  root_present[i] describes the i-th grade of the root mask, ascending: a bitmap of C(n,k)
+ * bits in gaast_batch_alloc_sparse's convention (bit c of word c / 64 = component c is stored), or NULL for the
+ * whole grade.  Normalised as a batch's bitmaps are: bits past C(n,k) are ignored, a grade with every bit set is
+ * dense, a grade with none stores nothing.  Selecting every component gives a plan indistinguishable from
+ * gaast_plan_create's.  A projection that stores no component at all is GAAST_ERR_SHAPE, a NULL root_present
+ * GAAST_ERR_INVALID; every other check is gaast_plan_create's.  ctx == NULL gives an offline plan (kernel_source /
+ * precompile then return and compile the projected kernels).
+ *   - gaast_eval / gaast_eval_sum accept only an output batch that matches: the same dimension, exactly the root grade
+ *     set, not broadcast, and per grade the same stored components (dense where the whole grade is selected).  Any
+ *     other output batch is GAAST_ERR_SHAPE, a dense one too when some grade is only partly selected.
+ *   - The kernels never compute a term that feeds only dropped components.  In GAAST_ARITH_STRICT each stored
+ *     component is bit-identical to the same component of the unprojected plan, on the specialised and the table
+ *     engine (every output keeps the reference's term order).
+ *   - gaast_eval_sum writes one double per STORED root component, in the output batch's stored-row order (grades
+ *     ascending, stored components ascending), with `out` present or NULL; an empty batch zeroes that many doubles.
+ *   - GAAST_ENGINE_DENSE_WARP is GAAST_ERR_UNSUPPORTED (AUTO never picks it for a projected plan), and so are
+ *     gaast_eval_host / _f32: their pipeline allocates dense output batches. */
+gaast_status gaast_plan_create_projected(gaast_ctx* ctx, const gaast_plan_desc* desc, const uint64_t* const* root_present,
+                                         gaast_plan** out);
 gaast_status gaast_plan_destroy(gaast_plan* plan);
 /* Algorithmic bytes and flops per batch element (SURVEY.md 8d), for f64 batches (f32: half the bytes): 8 x (f64 read
  * from non-broadcast inputs in the grades the plan reads + f64 written in the
- * root grades) and 2 x terms.  `broadcast_slots` bit s = slot s is broadcast. */
+ * root grades -- for a projected plan the stored root components only) and 2 x terms (the reference's terms: it has
+ * no projection, so a projected plan reports the flops of the whole expression).  `broadcast_slots` bit s = slot s
+ * is broadcast. */
 gaast_status gaast_plan_cost(const gaast_plan* plan, uint64_t broadcast_slots, uint64_t* bytes_per_elem,
                              uint64_t* flops_per_elem);
 uint32_t gaast_plan_root_mask(const gaast_plan* plan);
@@ -321,7 +344,7 @@ gaast_status gaast_eval(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n
 
 /* Batch-sum node (no reference definition: gaast has no batches): evaluates the
  * plan and reduces the root over the batch on the device, writing
- * sum_i out[i] as [root comps] f64 to `dev_sum` (device memory).  The
+ * sum_i out[i] as [root comps] f64 to `dev_sum` (device memory; a projected plan: [stored root comps]).  The
  * reduction is fused in the kernel epilogue; per-CTA partials are then added
  * in a fixed order, so the result is deterministic for a given launch shape.
  * `out` may be NULL to skip materialising the per-element result. */

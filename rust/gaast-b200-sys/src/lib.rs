@@ -128,6 +128,7 @@ extern "C" {
     pub fn gaast_ctx_launch_count(ctx: *mut gaast_ctx) -> u64;
 
     pub fn gaast_plan_create(ctx: *mut gaast_ctx, desc: *const gaast_plan_desc, out: *mut *mut gaast_plan) -> c_int;
+    pub fn gaast_plan_create_projected(ctx: *mut gaast_ctx, desc: *const gaast_plan_desc, root_present: *const *const u64, out: *mut *mut gaast_plan) -> c_int;
     pub fn gaast_plan_destroy(plan: *mut gaast_plan) -> c_int;
     pub fn gaast_plan_cost(plan: *const gaast_plan, broadcast_slots: u64, bytes_per_elem: *mut u64, flops_per_elem: *mut u64) -> c_int;
     pub fn gaast_plan_root_mask(plan: *const gaast_plan) -> u32;
