@@ -49,13 +49,6 @@ struct DeviceGuard {
     }
 };
 
-uint32_t rows_of(uint32_t n, uint32_t mask) {
-    uint32_t r = 0;
-    for (uint32_t k = 0; k <= n; ++k)
-        if (mask >> k & 1) r += uint32_t(gaast::binomial(n, k));
-    return r;
-}
-
 template <class T>
 void upload(T*& dst, const std::vector<T>& src, cudaStream_t s) {
     dst = nullptr;
@@ -162,6 +155,42 @@ void bind_streams(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_input
     a.total_cols = int(h.total_cols);
     a.root_col = int(h.buf_col[0]);
     a.store_out = out ? 1 : 0;
+}
+
+// The specialised kernel gaast_eval launches for a call; kernel_source and precompile name it through this function too.
+// A batch it cannot address with 128-bit accesses gets one element per thread and no TMA (bulk copies need 16-byte
+// aligned row segments).
+gaast::CodegenOptions specialized_options(const gaast_plan* plan, uint64_t broadcast_slots, int arith, bool with_sum,
+                                          bool store_out, bool f32, const std::vector<std::vector<uint64_t>>& sparse,
+                                          uint64_t sparse_hash, bool aligned) {
+    gaast::CodegenOptions opt;
+    opt.broadcast_slots = broadcast_slots;
+    opt.arith = arith;
+    opt.with_sum = with_sum;
+    opt.store_out = store_out;
+    opt.f32 = f32;
+    opt.sparse = sparse;
+    opt.sparse_hash = sparse_hash;
+    opt.variant = plan->variant;
+    opt.elems_per_thread = aligned ? plan->force_ept : 1;
+    // TMA-pipelined staging is opt-in (variant bit 3): measured slower than plain blocks on cfg3 / cfg5
+    opt.pipelined = aligned && (plan->variant & 8);
+    opt.tma_stage = aligned && !opt.pipelined && !with_sum && !(plan->variant & 1024);
+    return opt;
+}
+
+// A chain of geometric products runs on the dense engine's matrix-representation kernel unless variant bit 20 asks
+// for the term-by-term kernels.
+bool wants_matrix_kernel(const gaast_plan* plan, const gaast::DenseWarpHost& prog) { return prog.mat && !(plan->variant & 1048576); }
+
+// Generates and compiles (or finds in the cache) one kernel of the dense engine for a device of `dev`'s shape and a
+// batch of `batch` elements: the term-by-term kernel of product `step` with its signs folded at compile time, or for
+// step < 0 the matrix-representation kernel of the chain (dense_matrix.cu).  `*cg` receives its source.
+std::vector<char> build_dense(const gaast::DenseWarpHost& prog, const gaast_ctx& dev, long long batch, int step,
+                              gaast::CodegenResult* cg, std::string* key, std::string* origin, std::string* log) {
+    *cg = step >= 0 ? gaast::dense_warp_codegen(prog.n, prog.steps[size_t(step)].prod, gaast::dense_warp_shape(dev, prog.n, batch))
+                    : gaast::dense_matrix_codegen(*prog.mat, gaast::dense_matrix_shape(dev, *prog.mat, batch));
+    return gaast::jit_cubin(*cg, key, origin, log);
 }
 
 }  // namespace
@@ -366,29 +395,22 @@ static size_t kernel_source_impl(gaast_plan* plan, uint64_t broadcast_slots, int
     size_t len = 0;
     gaast_status st = guard([&] {
         if (!plan) throw Error(GAAST_ERR_INVALID, "null plan");
-        gaast::CodegenOptions opt;
-        opt.broadcast_slots = broadcast_slots;
-        opt.arith = arith;
-        opt.with_sum = (with_sum & GAAST_SRC_WITH_SUM) != 0;
-        opt.store_out = !(with_sum & GAAST_SRC_NO_STORE);
-        opt.f32 = (with_sum & GAAST_SRC_F32) != 0;
-        if (!opt.store_out && !opt.with_sum) throw Error(GAAST_ERR_INVALID, "kernel_source: a kernel that neither stores nor sums");
-        opt.elems_per_thread = plan->force_ept;
-        opt.variant = plan->variant;
-        // the kernel gaast_eval launches for an aligned batch (the same choices as eval_impl / precompile)
-        opt.pipelined = (opt.variant & 8) != 0;
-        opt.tma_stage = !opt.pipelined && !opt.with_sum && !(opt.variant & 1024);
+        const bool sum = (with_sum & GAAST_SRC_WITH_SUM) != 0, store = !(with_sum & GAAST_SRC_NO_STORE);
+        if (!store && !sum) throw Error(GAAST_ERR_INVALID, "kernel_source: a kernel that neither stores nor sums");
+        std::vector<std::vector<uint64_t>> sparse;
         if (present) {
             const gaast::DevicePlanHost& h = plan->h;
             if (n_present != h.n_in_streams) throw Error(GAAST_ERR_SHAPE, "kernel_source_sparse: one bitmap pointer per (slot, grade) the plan reads");
-            opt.sparse.resize(h.streams.size());
+            sparse.resize(h.streams.size());
             for (uint32_t i = 0; i < n_present; ++i) {
                 if (!present[i]) continue;
                 const size_t words = (size_t(h.streams[i].rows) + 63) / 64;
-                opt.sparse[i].assign(present[i], present[i] + words);
+                sparse[i].assign(present[i], present[i] + words);
             }
         }
-        gaast::CodegenResult cg = gaast::generate_kernel(plan->h, opt);
+        // the kernel gaast_eval launches for an aligned batch
+        gaast::CodegenResult cg = gaast::generate_kernel(
+            plan->h, specialized_options(plan, broadcast_slots, arith, sum, store, (with_sum & GAAST_SRC_F32) != 0, sparse, 0, true));
         len = cg.source.size();
         if (buf && cap) {
             const size_t ncopy = std::min(cap - 1, len);
@@ -417,56 +439,38 @@ gaast_status gaast_plan_precompile_typed(gaast_plan* plan, uint64_t broadcast_sl
                                          int dtype) {
     return guard([&] {
         if (!plan) throw Error(GAAST_ERR_INVALID, "null plan");
-        gaast::CodegenOptions opt;
-        opt.broadcast_slots = broadcast_slots;
-        opt.arith = arith;
-        opt.with_sum = with_sum != 0;
-        opt.store_out = store_out != 0;
-        opt.elems_per_thread = plan->force_ept;
-        opt.variant = plan->variant;
-        opt.pipelined = (opt.variant & 8) != 0;
-        opt.tma_stage = !opt.pipelined && !opt.with_sum && !(opt.variant & 1024);
-        opt.f32 = dtype == GAAST_F32;
+        const bool f32 = dtype == GAAST_F32;
+        auto options = [&](bool aligned) {
+            return specialized_options(plan, broadcast_slots, arith, with_sum != 0, store_out != 0, f32, {}, 0, aligned);
+        };
         gaast::CodegenResult cg;
         std::string key, origin;
         try {
-            gaast::build_specialized(plan->h, opt, &cg, &key, &origin);
+            gaast::build_specialized(plan->h, options(true), &cg, &key, &origin);
             // ... and the variant gaast_eval takes for a batch it cannot address with 128-bit accesses / TMA row copies (an
-            // odd length or a misaligned pointer in caller-owned memory): one element per thread, no TMA staging.  With both
-            // in the cache no shape of a shipped workload compiles at run time.
-            {
-                gaast::CodegenOptions un = opt;
-                un.elems_per_thread = 1;
-                un.pipelined = false;
-                un.tma_stage = false;
-                gaast::CodegenResult cg2;
-                std::string key2, origin2;
-                try {
-                    gaast::build_specialized(plan->h, un, &cg2, &key2, &origin2);
-                } catch (const Error&) {
-                    // (a plan whose unaligned form does not fit is evaluated by the table engine for such batches)
-                }
+            // odd length or a misaligned pointer in caller-owned memory).  With both in the cache no shape of a shipped
+            // workload compiles at run time.
+            try {
+                gaast::CodegenResult unaligned;
+                gaast::build_specialized(plan->h, options(false), &unaligned, nullptr, nullptr);
+            } catch (const Error&) {
+                // (a plan whose unaligned form does not fit is evaluated by the table engine for such batches)
             }
         } catch (const Error&) {
             // too large / too wide to specialise: a full high-dimensional product gets its dense-warp kernel instead
             gaast::DenseWarpHost dw;
-            if (opt.f32 || opt.with_sum || arith != GAAST_ARITH_FMA || plan->h.projected || !gaast::dense_warp_analyse(plan->h, &dw)) throw;
-            gaast_ctx fake;  // offline: the launch shape of a B200 (227 KB of shared memory per block, 148 SMs)
-            fake.sm_count = 148;
-            fake.smem_optin = 232448;
-            const gaast::DenseWarpLaunch shape = gaast::dense_warp_shape(fake, plan->h.n, 1 << 20);
-            for (const gaast::DenseWarpStep& step : dw.steps) {  // one kernel per product (equal tables share a cubin)
-                cg = gaast::dense_warp_codegen(plan->h.n, step.prod, shape);
-                std::string log;
-                gaast::jit_cubin(cg, &key, &origin, &log);
-            }
+            if (f32 || with_sum || arith != GAAST_ARITH_FMA || plan->h.projected || !gaast::dense_warp_analyse(plan->h, &dw)) throw;
+            gaast_ctx b200;  // offline: the launch shape of a B200 (227 KB of shared memory per block, 148 SMs)
+            b200.sm_count = 148;
+            b200.smem_optin = 232448;
+            for (size_t i = 0; i < dw.steps.size(); ++i)  // one kernel per product (equal tables share a cubin)
+                build_dense(dw, b200, 1 << 20, int(i), &cg, &key, &origin, nullptr);
             cg.notes += " x" + std::to_string(dw.steps.size()) + " product(s)";
-            if (dw.mat && !(plan->variant & 1048576)) {  // a chain of geometric products: its matrix-representation kernel
+            if (wants_matrix_kernel(plan, dw)) {
                 const std::string dw_notes = cg.notes;
-                cg = gaast::dense_matrix_codegen(*dw.mat, gaast::dense_matrix_shape(fake, *dw.mat, 1 << 20));
-                cg.notes = dw_notes + " " + cg.notes;
                 std::string log;
-                gaast::jit_cubin(cg, &key, &origin, &log);
+                build_dense(dw, b200, 1 << 20, -1, &cg, &key, &origin, &log);
+                cg.notes = dw_notes + " " + cg.notes;
                 const size_t used = log.find("Used ", log.find("Function properties for " + cg.kernel_name));
                 if (used != std::string::npos)
                     cg.notes += " regs=" + std::to_string(std::atoi(log.c_str() + used + 5)) +
@@ -802,9 +806,7 @@ gaast_status gaast_batch_download_records(const gaast_batch* b, uint64_t first, 
 
 // ---------------------------------------------------------------- eval ----
 static std::shared_ptr<gaast::JitKernel> get_specialized(gaast_plan* plan, const gaast::CodegenOptions& opt) {
-    auto key = std::make_tuple(opt.broadcast_slots, opt.arith, int(opt.with_sum), int(opt.store_out),
-                               opt.elems_per_thread, opt.variant, int(opt.pipelined), int(opt.tma_stage), int(opt.f32),
-                               opt.sparse_hash);
+    const gaast_plan::JitKey key = opt.key();
     auto it = plan->jit.find(key);
     if (it != plan->jit.end()) {
         // a negative entry: THIS variant failed to build before (other variants of the plan are unaffected)
@@ -828,6 +830,307 @@ static std::shared_ptr<gaast::JitKernel> get_specialized(gaast_plan* plan, const
     }
 }
 
+// build_dense's kernel for n elements on the plan's device, loaded once per launch shape (the matrix kernel is shared by
+// every signature of its shape).  Null when it is not wanted or cannot be built (never tried again for the plan): for a
+// product, the dense-warp engine then runs the generic kernel compiled into the library.
+static std::shared_ptr<gaast::JitKernel> dense_kernel(gaast_plan* plan, long long n, int step) {
+    const gaast::DenseWarpHost& prog = plan->dense_warp;
+    std::shared_ptr<gaast::JitKernel>* slot;
+    if (step >= 0) {
+        if (plan->dw_jit_failed || gaast::tuning().dense_warp_generic) return nullptr;
+        slot = &plan->dw_jit[std::make_pair(step, gaast::dense_warp_shape(*plan->ctx, prog.n, n).threads)];
+    } else {
+        if (!wants_matrix_kernel(plan, prog) || plan->dm_jit_failed) return nullptr;
+        const gaast::DenseMatLaunch s = gaast::dense_matrix_shape(*plan->ctx, *prog.mat, n);
+        slot = &plan->dm_jit[s.RC * 4194304 + s.threads * 8192 + s.T * 64 + s.blocks_per_sm * 4 + int(s.pipe) * 2 + int(s.csep)];
+    }
+    if (*slot) return *slot;
+    try {
+        gaast::CodegenResult cg;
+        std::string key, origin;
+        const std::vector<char> cubin = build_dense(prog, *plan->ctx, n, step, &cg, &key, &origin, nullptr);
+        auto k = gaast::jit_load(cg, cubin);
+        k->key = key;
+        k->origin = origin;
+        k->fma_per_elem = cg.fma_per_elem;
+        return *slot = k;
+    } catch (const Error&) {
+        (step >= 0 ? plan->dw_jit_failed : plan->dm_jit_failed) = true;
+        return nullptr;
+    }
+}
+
+// One gaast_eval call, validated and bound to its batches (bind_streams).
+struct EvalCall {
+    gaast_plan* plan;
+    gaast_batch* out;  // null: sums only
+    int arith;
+    bool with_sum, f32 = false;
+    gaast::EvalArgs a{};
+    uint64_t bslots = 0;  // broadcast input slots
+    long long n = 0;
+    std::vector<std::vector<uint64_t>> sparse{};  // the inputs' stored components, and a hash of them
+    uint64_t sparse_hash = 0;
+};
+
+// Whether the dense-warp engine can evaluate the call: a chain of dense products, f64, FMA arithmetic, per-element
+// operands.  The first call analyses the plan and uploads its tables.
+static bool dense_warp_ready(EvalCall& c) {
+    gaast_plan* plan = c.plan;
+    const gaast::DevicePlanHost& h = plan->h;
+    if (c.with_sum || c.f32 || c.arith != GAAST_ARITH_FMA || !c.out) return false;
+    if (plan->dense_warp_state == 0) {
+        plan->dense_warp_state = gaast::dense_warp_analyse(h, &plan->dense_warp) ? 1 : -1;
+        if (plan->dense_warp_state == 1) {
+            upload(plan->d_dw_blades, plan->dense_warp.blade_of_slot, plan->ctx->stream);
+            if (plan->dense_warp.mat) {
+                upload(plan->d_dm_src, gaast::matrix_rep_device_table(*plan->dense_warp.mat), plan->ctx->stream);
+                upload(plan->d_dm_lx, plan->dense_warp.mat->lx, plan->ctx->stream);
+                cuda_check(cudaMalloc(&plan->d_dm_rows, ((size_t(3) << h.n) + (size_t(3) << plan->dense_warp.mat->mx)) *
+                                                            sizeof(unsigned long long)),  // row addresses + flag words
+                           "cudaMalloc(dense-matrix row tables)");
+            }
+        }
+    }
+    if (plan->dense_warp_state != 1) return false;
+    if (h.n > 10 && !dense_kernel(plan, c.n, -1)) return false;  // no term-by-term kernel above n = 10: the matrix kernel or nothing
+    // products that drop pairs (outer products, contractions) need their per-plan kernel
+    for (size_t i = 0; i < plan->dense_warp.steps.size() && !plan->dense_warp.complete; ++i)
+        if (!plan->dense_warp.steps[i].prod.complete && !dense_kernel(plan, c.n, int(i))) return false;
+    return true;
+}
+
+// The launch length of the specialised kernel and whether it can address the batch with 128-bit accesses: every
+// per-element row 16-byte aligned and as long as the launch, every stride a whole number of 16 bytes.  An odd-length
+// batch (the ragged tail of a chunked run) still takes the aligned kernel when the library owns the output batch: rows
+// are padded to 128 bytes, so the launch simply covers the padding column(s) too.  Inputs are only read there;
+// caller-owned (wrapped) outputs are never written beyond their length, and a batch-sum must not see the padding.
+struct LaunchLength { bool aligned; long long n; };
+static LaunchLength launch_length(const EvalCall& c) {
+    const gaast::DevicePlanHost& h = c.plan->h;
+    const long long quantum = c.f32 ? 4 : 2;  // elements per 16 bytes
+    auto rows_fit = [&](long long len) {
+        for (size_t i = 0; i < h.streams.size(); ++i) {
+            if ((c.a.bcast[i >> 6] >> (i & 63) & 1) || !c.a.sptr[i]) continue;  // (broadcast operands: one element)
+            if (c.a.srow[i] < len || (c.a.srow[i] % quantum) || (reinterpret_cast<uintptr_t>(c.a.sptr[i]) & 15)) return false;
+        }
+        return true;
+    };
+    if (c.n % quantum == 0) return {rows_fit(c.n), c.n};
+    const long long padded = (c.n + quantum - 1) / quantum * quantum;
+    if (!c.with_sum && (!c.out || c.out->owned) && rows_fit(padded)) return {true, padded};
+    return {false, c.n};
+}
+
+enum class Engine { dense_warp, specialized, table };
+
+// Which engine evaluates the call; `*jk` receives the specialised kernel.  AUTO takes the specialised kernel, else a
+// dense enough product's dense-warp engine, else the table engine.
+static Engine choose_engine(EvalCall& c, int engine, std::shared_ptr<gaast::JitKernel>* jk) {
+    const gaast::DevicePlanHost& h = c.plan->h;
+    if (engine == GAAST_ENGINE_DENSE_WARP) {
+        if (h.projected)
+            throw Error(GAAST_ERR_UNSUPPORTED, "dense-warp engine: a projected plan is evaluated by the specialised or the "
+                                               "table engine");
+        if (!dense_warp_ready(c))
+            throw Error(GAAST_ERR_UNSUPPORTED,
+                        "dense-warp engine: the plan is not a chain of dense products (geometric, outer, contraction) of "
+                        "full-grade per-element f64 operands in G(n), 7 <= n <= 10, with a +-1 metric, evaluated in FMA "
+                        "arithmetic without batch-sum");
+        return Engine::dense_warp;
+    }
+    if (engine == GAAST_ENGINE_TABLE) return Engine::table;
+    if (engine != GAAST_ENGINE_AUTO && engine != GAAST_ENGINE_SPECIALIZED) throw Error(GAAST_ERR_INVALID, "unknown engine");
+    // AUTO: a handful of elements of a plan never specialised before is not worth generating and
+    // compiling a kernel for (0.3-3 s): the table engine evaluates it at once.
+    const bool any_sparse = !c.sparse.empty();
+    if (engine == GAAST_ENGINE_AUTO && c.plan->jit.empty() && !any_sparse &&
+        double(c.n) * double(h.total_terms > 0 ? h.total_terms : 1) < 2e6)
+        return Engine::table;
+    // (a batch widened over the output's padding stays widened for the engine that takes over below)
+    const LaunchLength len = launch_length(c);
+    c.n = c.a.n = len.n;
+    try {
+        *jk = get_specialized(c.plan, specialized_options(c.plan, c.bslots, c.arith, c.with_sum, c.out != nullptr, c.f32,
+                                                          c.sparse, c.sparse_hash, len.aligned));
+        return Engine::specialized;
+    } catch (const Error&) {
+        // AUTO: this variant cannot be specialised (too large, or no NVRTC and no cached cubin): another engine
+        // evaluates it.  The failure is remembered per variant (get_specialized), so an odd-length call that needs
+        // another kernel does not take the fast path away from aligned calls.
+        if (engine == GAAST_ENGINE_SPECIALIZED || any_sparse) throw;  // (no other engine reads a sparse batch)
+    }
+    // too large / too wide to specialise: a full high-dimensional product still has a fast engine
+    // (the engine always runs COMPLETE 4^n products.  Measured per kept pair: 12-15 TFLOP/s against 1.2-2.1 on
+    // the table engine at n = 7, 8 -- worth it while the plan keeps at least 1/8 of the pairs; at n = 9, 10 the
+    // table engine's workspace is in global memory (0.09 TFLOP/s): 1/64.  exp/rotor_square.py, exp/big_products.py)
+    const double min_density = h.n <= 8 ? 1.0 / 8.0 : 1.0 / 64.0;
+    if (!h.projected && dense_warp_ready(c) &&
+        double(h.total_terms) >= min_density * double(c.plan->dense_warp.steps.size()) * std::pow(4.0, double(h.n)))
+        return Engine::dense_warp;
+    return Engine::table;
+}
+
+// Points a batch-sum kernel at the plan's partials, sized for the largest grid its engine can launch for the plan so
+// that only the first call allocates.
+static void bind_partials(EvalCall& c, size_t max_grid) {
+    if (!c.with_sum) return;
+    ensure(c.plan->d_partials, c.plan->partials_cap, (max_grid + gaast::kReduceStage1Rows) * size_t(c.a.n_sum_cols));
+    c.a.partials = c.plan->d_partials;
+}
+
+// Each launcher enqueues its engine's kernels, describes them in last_kernel and returns the grid it launched.
+static int launch_dense_warp(EvalCall& c) {
+    gaast_plan* plan = c.plan;
+    gaast_ctx* ctx = plan->ctx;
+    const gaast::DevicePlanHost& h = plan->h;
+    const gaast::DenseWarpHost& prog = plan->dense_warp;
+    const long long n = c.n;
+    // scratch buffers for the intermediate products: [2^n][stride], rows on 128-byte boundaries
+    const size_t stride = (size_t(n) + 15) / 16 * 16;
+    if (plan->d_dw_scratch.size() < size_t(prog.n_scratch) || plan->dw_scratch_stride < stride) {
+        for (double* p : plan->d_dw_scratch) cudaFree(p);
+        plan->d_dw_scratch.assign(size_t(prog.n_scratch), nullptr);
+        plan->dw_scratch_stride = 0;
+        for (double*& p : plan->d_dw_scratch)
+            cuda_check(cudaMalloc(&p, (size_t(1) << h.n) * stride * sizeof(double)), "cudaMalloc(dense-warp scratch)");
+        plan->dw_scratch_stride = stride;
+    }
+    auto buffers_of = [&](const gaast::DenseWarpOperand& o) {
+        gaast::DenseWarpBuffers b;
+        size_t root_stream = h.n_in_streams;  // the root's grade arrays follow the inputs, grades ascending
+        for (uint32_t k = 0; k <= h.n; ++k) {
+            if (!(o.grade_mask >> k & 1)) continue;  // no data / not stored: the kernel never touches it
+            if (o.slot >= 0) {
+                const int si = h.stream_of(uint32_t(o.slot), k);
+                if (si < 0) throw Error(GAAST_ERR_INVALID, "dense-warp engine: the plan has no stream for a grade it reads");
+                b.ptr[k] = c.a.sptr[si];
+                b.row[k] = c.a.srow[si];
+                b.shared = (c.bslots >> o.slot) & 1;  // a fixed operand (the rotor of R X ~R): stride 0
+            } else if (o.root) {
+                b.ptr[k] = c.a.sptr[root_stream];
+                b.row[k] = c.a.srow[root_stream];
+                ++root_stream;
+            } else {
+                b.ptr[k] = plan->d_dw_scratch[size_t(o.scratch)] + size_t(prog.gstart[k]) * plan->dw_scratch_stride;
+                b.row[k] = (long long)plan->dw_scratch_stride;
+            }
+        }
+        return b;
+    };
+    if (std::shared_ptr<gaast::JitKernel> dmk = dense_kernel(plan, n, -1)) {
+        const gaast::DenseMatLaunch mshape = gaast::dense_matrix_shape(*ctx, *prog.mat, n);
+        for (const gaast::DenseWarpStep& step : prog.steps) {
+            cuda_check(gaast::dense_matrix_launch(prog, step, buffers_of(step.L), buffers_of(step.R), buffers_of(step.O),
+                                                  step.C.slot >= 0 ? buffers_of(step.C) : gaast::DenseWarpBuffers(), n,
+                                                  plan->d_dm_src, plan->d_dm_lx, plan->d_dm_rows, mshape,
+                                                  dmk->kernel, ctx->stream),
+                       "launch dense-matrix kernel");
+            ctx->launches += 2;  // the row-address prologue and the product
+        }
+        char desc[400];
+        std::snprintf(desc, sizeof desc,
+                      "gaast_dense_matrix engine=dense_warp kernel=matrix origin=%s products=%zu grid=%d block=%d smem=%zu "
+                      "tile=%d elements regs=%d spill=%zuB blocks/SM=%d fma/elem=%d key=%s M%d x%d cols=%d",
+                      dmk->origin.c_str(), prog.steps.size(), mshape.grid, mshape.threads, mshape.smem, mshape.T, dmk->regs,
+                      dmk->local_bytes, mshape.blocks_per_sm, dmk->fma_per_elem, dmk->key.c_str(), 1 << prog.mat->mx,
+                      1 << prog.mat->db, 1 << prog.mat->dl);
+        plan->last_kernel = desc;
+        return mshape.grid;
+    }
+    const gaast::DenseWarpLaunch shape = gaast::dense_warp_shape(*ctx, h.n, n);
+    std::shared_ptr<gaast::JitKernel> dwk;
+    for (size_t i = 0; i < prog.steps.size(); ++i) {
+        const gaast::DenseWarpStep& step = prog.steps[i];
+        dwk = dense_kernel(plan, n, int(i));
+        cuda_check(gaast::dense_warp_launch(prog, step, buffers_of(step.L), buffers_of(step.R), buffers_of(step.O),
+                                            step.C.slot >= 0 ? buffers_of(step.C) : gaast::DenseWarpBuffers(), n,
+                                            plan->d_dw_blades, shape, dwk ? dwk->kernel : nullptr, ctx->stream),
+                   "launch dense-warp engine");
+        ctx->launches++;
+    }
+    char desc[320];
+    std::snprintf(desc, sizeof desc,
+                  "%s engine=dense_warp origin=%s products=%zu grid=%d block=%d smem=%zu tile=%d elements regs=%d",
+                  dwk ? "gaast_dense_warp" : "dense_warp_kernel", dwk ? dwk->origin.c_str() : "library",
+                  prog.steps.size(), shape.grid, shape.threads, shape.smem, shape.T, dwk ? dwk->regs : 0);
+    plan->last_kernel = desc;
+    return shape.grid;
+}
+
+static int launch_specialized(EvalCall& c, const gaast::JitKernel& jk) {
+    gaast_ctx* ctx = c.plan->ctx;
+    const long long per_block = (long long)jk.threads * jk.elems_per_thread;
+    const long long blocks = (c.n + per_block - 1) / per_block;
+    if (blocks > 0x7fffffffLL) throw Error(GAAST_ERR_SHAPE, "batch too long for one launch");
+    int grid = int(blocks);
+    size_t max_grid = size_t(grid);
+    if ((c.with_sum || jk.pipelined || gaast::tuning().force_persistent) && !jk.one_tile_blocks) {
+        // persistent grid: the batch-sum epilogue keeps per-block partials, and the TMA-pipelined
+        // kernels loop over their tiles; blocks stride over the batch
+        // sum-only kernels: many short-lived blocks overlap better than one long-lived block per resident slot, but
+        // every block pays its epilogue (column sums -> partials), so a block should still see ~8 tiles.  Measured
+        // on cfg5 + sum (ms per step at 4 / 8 / 16 / 32 / 64 blocks per slot): 32 M elements 6.42 / 6.20 / - / 5.97 /
+        // 5.92; 8 M (the 4-GPU shard) 1.577 / 1.535 / 1.505 / 1.501 / 1.558; 4 M (the 8-GPU shard) 0.787 / 0.770 /
+        // 0.770 / 0.793 / 0.857.
+        const long long resident = (long long)ctx->sm_count * jk.blocks_per_sm;
+        long long mult = jk.pipelined ? 1 : std::min(64LL, std::max(4LL, blocks / (8 * resident)));
+        if (gaast::tuning().grid_mult > 0) mult = gaast::tuning().grid_mult;
+        const long long cap = resident * mult;
+        if (grid > cap) grid = int(cap);
+        max_grid = size_t(resident * std::max(64LL, mult));  // (>= the capped grid of every call of this variant)
+    }
+    bind_partials(c, max_grid);
+    if (jk.n_uniform > 0) {
+        ensure(c.plan->d_uniform, c.plan->uniform_cap, size_t(jk.n_uniform));
+        c.a.uniform = c.plan->d_uniform;
+        void* params[] = {&c.a};
+        cuda_check(cudaLaunchKernel(reinterpret_cast<const void*>(jk.uniform_kernel), dim3(1), dim3(32), params, 0,
+                                    ctx->stream),
+                   "launch uniform prologue");
+        ctx->launches++;
+    }
+    c.a.lookahead = ctx->sm_count * jk.blocks_per_sm;  // resident blocks: the look-ahead distance of the L2 prefetch variant
+    if (gaast::tuning().lookahead >= 0) c.a.lookahead = gaast::tuning().lookahead;
+    void* params[] = {&c.a};
+    cuda_check(cudaLaunchKernel(reinterpret_cast<const void*>(jk.kernel), dim3(grid), dim3(jk.threads), params, jk.smem_bytes,
+                                ctx->stream),
+               "launch specialised kernel");
+    ctx->launches++;
+    char desc[512];
+    std::snprintf(desc, sizeof desc,
+                  "%s engine=specialized origin=%s grid=%d block=%d elems/thread=%d regs=%d spill=%zuB fma/elem=%d key=%s",
+                  jk.name.c_str(), jk.origin.c_str(), grid, jk.threads, jk.elems_per_thread, jk.regs, jk.local_bytes,
+                  jk.fma_per_elem, jk.key.c_str());
+    c.plan->last_kernel = desc;
+    return grid;
+}
+
+static int launch_table(EvalCall& c) {
+    gaast_plan* plan = c.plan;
+    gaast_ctx* ctx = plan->ctx;
+    const gaast::TableLaunch shape = gaast::table_engine_shape(*ctx, plan->h, c.n, c.with_sum, c.f32);
+    // scratch is sized for the largest grid the engine ever launches (8 blocks per SM)
+    const size_t max_grid = std::max(size_t(shape.grid), size_t(ctx->sm_count) * 8);
+    if (shape.global_ws) {
+        ensure(plan->d_ws, plan->ws_cap, max_grid * shape.ws_doubles_per_block);
+        c.a.ws_global = plan->d_ws;
+    }
+    bind_partials(c, max_grid);
+    c.a.micro = plan->d_micro;
+    c.a.chunks = plan->d_chunks;
+    c.a.n_micro = int(plan->h.micro.size());
+    c.a.n_chunks = int(plan->h.chunks.size());
+    cuda_check(gaast::table_engine_launch(c.a, shape, c.arith == GAAST_ARITH_STRICT, c.with_sum, c.f32, ctx->stream),
+               "launch table engine");
+    ctx->launches++;
+    char desc[256];
+    std::snprintf(desc, sizeof desc, "table_engine_kernel engine=table grid=%d block=%d smem=%zu ws=%s", shape.grid,
+                  shape.threads, shape.smem, shape.global_ws ? "global" : "shared");
+    plan->last_kernel = desc;
+    return shape.grid;
+}
+
 static void eval_impl(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_inputs, gaast_batch* out, double* dev_sum,
                       bool with_sum, int engine, int arith) {
     if (!plan) throw Error(GAAST_ERR_INVALID, "null plan");
@@ -836,334 +1139,23 @@ static void eval_impl(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_i
     if (arith != GAAST_ARITH_FMA && arith != GAAST_ARITH_STRICT) throw Error(GAAST_ERR_INVALID, "unknown arith mode");
     if (with_sum && !dev_sum) throw Error(GAAST_ERR_INVALID, "eval_sum: null sum pointer");
     DeviceGuard dg(ctx->device);
-    gaast::EvalArgs a;
-    uint64_t bslots = 0;
-    long long n = 0;
+    EvalCall c{plan, out, arith, with_sum};
     int dtype = GAAST_F64;
-    std::vector<std::vector<uint64_t>> sparse;
-    uint64_t sparse_hash = 0;
-    bind_streams(plan, inputs, n_inputs, out, !with_sum, a, &bslots, &n, &dtype, &sparse, &sparse_hash);
-    const bool any_sparse = !sparse.empty();
-    if (any_sparse && (engine == GAAST_ENGINE_TABLE || engine == GAAST_ENGINE_DENSE_WARP))
+    bind_streams(plan, inputs, n_inputs, out, !with_sum, c.a, &c.bslots, &c.n, &dtype, &c.sparse, &c.sparse_hash);
+    c.f32 = dtype == GAAST_F32;
+    if (!c.sparse.empty() && (engine == GAAST_ENGINE_TABLE || engine == GAAST_ENGINE_DENSE_WARP))
         throw Error(GAAST_ERR_UNSUPPORTED, "sparse batches are evaluated by the specialised engine only (the kernel is "
                                            "generated for the sparsity pattern): use GAAST_ENGINE_AUTO or GAAST_ENGINE_SPECIALIZED");
-    const bool f32 = dtype == GAAST_F32;
-    const gaast::DevicePlanHost& h = plan->h;
-    const int sum_cols = int(h.stored_cols);  // one column per stored root component
-    a.n_sum_cols = with_sum ? sum_cols : 0;
-    if (n == 0) {
+    const int sum_cols = int(plan->h.stored_cols);  // one column per stored root component
+    c.a.n_sum_cols = with_sum ? sum_cols : 0;
+    if (c.n == 0) {
         if (with_sum) cuda_check(cudaMemsetAsync(dev_sum, 0, sum_cols * sizeof(double), ctx->stream), "zero sum");
         return;
     }
-
-    // dense-warp engine: the per-plan kernel (warp-uniform signs folded at compile time) when NVRTC or the
-    // cache has it, else null = the generic kernel compiled into the library
-    auto dense_warp_kernel_for = [&](int step, const gaast::DenseWarpLaunch& shape) -> std::shared_ptr<gaast::JitKernel> {
-        if (plan->dw_jit_failed || gaast::tuning().dense_warp_generic) return nullptr;
-        const auto jkey = std::make_pair(step, shape.threads);
-        auto it = plan->dw_jit.find(jkey);
-        if (it != plan->dw_jit.end()) return it->second;
-        try {
-            gaast::CodegenResult cg = gaast::dense_warp_codegen(h.n, plan->dense_warp.steps[size_t(step)].prod, shape);
-            std::string key, origin, log;
-            std::vector<char> cubin = gaast::jit_cubin(cg, &key, &origin, &log);
-            auto k = gaast::jit_load(cg, cubin);
-            k->key = key;
-            k->origin = origin;
-            plan->dw_jit.emplace(jkey, k);
-            return k;
-        } catch (const Error&) {
-            plan->dw_jit_failed = true;
-            return nullptr;
-        }
-    };
-    // ... and the matrix-representation kernel of a chain of geometric products (dense_matrix.cu): one per tile shape,
-    // shared by every signature of that shape; null when it is switched off (variant bit 20) or cannot be built
-    auto dense_matrix_kernel_for = [&](const gaast::DenseMatLaunch& shape) -> std::shared_ptr<gaast::JitKernel> {
-        if (!plan->dense_warp.mat || plan->dm_jit_failed || (plan->variant & 1048576)) return nullptr;
-        auto it = plan->dm_jit.find(shape.RC * 4194304 + shape.threads * 8192 + shape.T * 64 + shape.blocks_per_sm * 4 + int(shape.pipe) * 2 + int(shape.csep));
-        if (it != plan->dm_jit.end()) return it->second;
-        try {
-            gaast::CodegenResult cg = gaast::dense_matrix_codegen(*plan->dense_warp.mat, shape);
-            std::string key, origin, log;
-            std::vector<char> cubin = gaast::jit_cubin(cg, &key, &origin, &log);
-            auto k = gaast::jit_load(cg, cubin);
-            k->key = key;
-            k->origin = origin;
-            k->fma_per_elem = cg.fma_per_elem;
-            plan->dm_jit.emplace(shape.RC * 4194304 + shape.threads * 8192 + shape.T * 64 + shape.blocks_per_sm * 4 + int(shape.pipe) * 2 + int(shape.csep), k);
-            return k;
-        } catch (const Error&) {
-            plan->dm_jit_failed = true;
-            return nullptr;
-        }
-    };
-    // usable for this call?  (a chain of dense products, f64, FMA arithmetic, per-element operands)
-    auto dense_warp_ready = [&]() {
-        if (with_sum || f32 || arith != GAAST_ARITH_FMA || !out) return false;
-        if (plan->dense_warp_state == 0) {
-            plan->dense_warp_state = gaast::dense_warp_analyse(h, &plan->dense_warp) ? 1 : -1;
-            if (plan->dense_warp_state == 1) {
-                upload(plan->d_dw_blades, plan->dense_warp.blade_of_slot, ctx->stream);
-                if (plan->dense_warp.mat) {
-                    upload(plan->d_dm_src, gaast::matrix_rep_device_table(*plan->dense_warp.mat), ctx->stream);
-                    upload(plan->d_dm_lx, plan->dense_warp.mat->lx, ctx->stream);
-                    cuda_check(cudaMalloc(&plan->d_dm_rows, ((size_t(3) << h.n) + (size_t(3) << plan->dense_warp.mat->mx)) *
-                                                                sizeof(unsigned long long)),  // row addresses + flag words
-                               "cudaMalloc(dense-matrix row tables)");
-                }
-            }
-        }
-        if (plan->dense_warp_state != 1) return false;
-        if (h.n > 10 &&  // no term-by-term kernel above n = 10: the matrix kernel or nothing
-            !(plan->dense_warp.mat && dense_matrix_kernel_for(gaast::dense_matrix_shape(*ctx, *plan->dense_warp.mat, n))))
-            return false;
-        // products that drop pairs (outer products, contractions) need their per-plan kernel
-        if (!plan->dense_warp.complete) {
-            const gaast::DenseWarpLaunch shape = gaast::dense_warp_shape(*ctx, h.n, n);
-            for (size_t i = 0; i < plan->dense_warp.steps.size(); ++i)
-                if (!plan->dense_warp.steps[i].prod.complete && !dense_warp_kernel_for(int(i), shape)) return false;
-        }
-        return true;
-    };
-    bool use_dense_warp = false;
-    if (engine == GAAST_ENGINE_DENSE_WARP && h.projected)
-        throw Error(GAAST_ERR_UNSUPPORTED, "dense-warp engine: a projected plan is evaluated by the specialised or the "
-                                           "table engine");
-    if (engine == GAAST_ENGINE_DENSE_WARP) {
-        if (!dense_warp_ready())
-            throw Error(GAAST_ERR_UNSUPPORTED,
-                        "dense-warp engine: the plan is not a chain of dense products (geometric, outer, contraction) of "
-                        "full-grade per-element f64 operands in G(n), 7 <= n <= 10, with a +-1 metric, evaluated in FMA "
-                        "arithmetic without batch-sum");
-        use_dense_warp = true;
-    }
-
     std::shared_ptr<gaast::JitKernel> jk;
-    // AUTO: a handful of elements of a plan never specialised before is not worth generating and
-    // compiling a kernel for (0.3-3 s): the table engine evaluates it at once.
-    const bool tiny = engine == GAAST_ENGINE_AUTO && plan->jit.empty() && !any_sparse &&
-                      double(n) * double(h.total_terms > 0 ? h.total_terms : 1) < 2e6;
-    if (use_dense_warp) {
-        // chosen explicitly
-    } else if ((engine == GAAST_ENGINE_AUTO && !tiny) || engine == GAAST_ENGINE_SPECIALIZED) {
-        {
-            try {
-                gaast::CodegenOptions opt;
-                opt.broadcast_slots = bslots;
-                opt.arith = arith;
-                opt.with_sum = with_sum;
-                opt.store_out = out != nullptr;
-                opt.elems_per_thread = plan->force_ept;
-                opt.variant = plan->variant;
-                opt.f32 = f32;
-                opt.sparse = sparse;
-                opt.sparse_hash = sparse_hash;
-                // 128-bit accesses need even strides and 16-byte aligned rows
-                const long long quantum = f32 ? 4 : 2;  // elements per 16 bytes
-                bool aligned = (n % quantum == 0);
-                for (size_t i = 0; i < h.streams.size(); ++i) {
-                    const bool bc = (a.bcast[i >> 6] >> (i & 63)) & 1;
-                    if (bc || !a.sptr[i]) continue;
-                    if ((a.srow[i] % quantum) || (reinterpret_cast<uintptr_t>(a.sptr[i]) & 15)) aligned = false;
-                }
-                // An odd-length batch (the ragged tail of a chunked run) still takes the aligned kernel when the
-                // library owns the output batch: rows are padded to 128 bytes, so the launch simply covers the
-                // padding column(s) too.  Inputs are only read there; caller-owned (wrapped) outputs are never
-                // written beyond their length, and a batch-sum must not see the padding.
-                if (!aligned && !with_sum && (!out || out->owned) && n % quantum != 0) {
-                    const long long padded = (n + quantum - 1) / quantum * quantum;
-                    bool fits = true;
-                    for (size_t i = 0; i < h.streams.size(); ++i) {
-                        const bool bc = (a.bcast[i >> 6] >> (i & 63)) & 1;
-                        if (bc || !a.sptr[i]) continue;
-                        if (a.srow[i] < padded || (a.srow[i] % quantum) || (reinterpret_cast<uintptr_t>(a.sptr[i]) & 15)) fits = false;
-                    }
-                    if (fits) {
-                        aligned = true;
-                        n = padded;
-                        a.n = padded;
-                    }
-                }
-                if (!aligned) opt.elems_per_thread = 1;
-                // TMA-pipelined staging is opt-in (variant bit 3): measured slower than plain blocks on cfg3 / cfg5
-                opt.pipelined = aligned && (opt.variant & 8);  // TMA bulk copies need 16-byte aligned row segments
-                opt.tma_stage = aligned && !opt.pipelined && !with_sum && !(opt.variant & 1024);
-                jk = get_specialized(plan, opt);
-            } catch (const Error&) {
-                // AUTO: this variant cannot be specialised (too large, or no NVRTC and no cached cubin): the table
-                // engine evaluates it.  The failure is remembered per variant (get_specialized), so an odd-length
-                // call that needs another kernel does not take the fast path away from aligned calls.
-                if (engine == GAAST_ENGINE_SPECIALIZED || any_sparse) throw;  // (no other engine reads a sparse batch)
-            }
-        }
-        // too large / too wide to specialise: a full high-dimensional product still has a fast engine
-        // (the engine always runs COMPLETE 4^n products.  Measured per kept pair: 12-15 TFLOP/s against 1.2-2.1 on
-        // the table engine at n = 7, 8 -- worth it while the plan keeps at least 1/8 of the pairs; at n = 9, 10 the
-        // table engine's workspace is in global memory (0.09 TFLOP/s): 1/64.  exp/rotor_square.py, exp/big_products.py)
-        const double min_density = h.n <= 8 ? 1.0 / 8.0 : 1.0 / 64.0;
-        if (!jk && engine == GAAST_ENGINE_AUTO && !h.projected && dense_warp_ready() &&
-            double(h.total_terms) >= min_density * double(plan->dense_warp.steps.size()) * std::pow(4.0, double(h.n)))
-            use_dense_warp = true;
-    } else if (engine != GAAST_ENGINE_TABLE && engine != GAAST_ENGINE_AUTO) {
-        throw Error(GAAST_ERR_INVALID, "unknown engine");
-    }
-
-    int grid = 0;
-    if (use_dense_warp) {
-        const gaast::DenseWarpLaunch shape = gaast::dense_warp_shape(*ctx, h.n, n);
-        grid = shape.grid;
-        const gaast::DenseWarpHost& prog = plan->dense_warp;
-        // scratch buffers for the intermediate products: [2^n][stride], rows on 128-byte boundaries
-        const size_t stride = (size_t(n) + 15) / 16 * 16;
-        if (plan->d_dw_scratch.size() < size_t(prog.n_scratch) || plan->dw_scratch_stride < stride) {
-            for (double* p : plan->d_dw_scratch) cudaFree(p);
-            plan->d_dw_scratch.assign(size_t(prog.n_scratch), nullptr);
-            plan->dw_scratch_stride = 0;
-            for (double*& p : plan->d_dw_scratch)
-                cuda_check(cudaMalloc(&p, (size_t(1) << h.n) * stride * sizeof(double)), "cudaMalloc(dense-warp scratch)");
-            plan->dw_scratch_stride = stride;
-        }
-        auto buffers_of = [&](const gaast::DenseWarpOperand& o) {
-            gaast::DenseWarpBuffers b;
-            size_t root_stream = h.n_in_streams;  // the root's grade arrays follow the inputs, grades ascending
-            for (uint32_t k = 0; k <= h.n; ++k) {
-                if (!(o.grade_mask >> k & 1)) continue;  // no data / not stored: the kernel never touches it
-                if (o.slot >= 0) {
-                    const int si = h.stream_of(uint32_t(o.slot), k);
-                    if (si < 0) throw Error(GAAST_ERR_INVALID, "dense-warp engine: the plan has no stream for a grade it reads");
-                    b.ptr[k] = a.sptr[si];
-                    b.row[k] = a.srow[si];
-                    b.shared = (bslots >> o.slot) & 1;  // a fixed operand (the rotor of R X ~R): stride 0
-                } else if (o.root) {
-                    b.ptr[k] = a.sptr[root_stream];
-                    b.row[k] = a.srow[root_stream];
-                    ++root_stream;
-                } else {
-                    b.ptr[k] = plan->d_dw_scratch[size_t(o.scratch)] + size_t(prog.gstart[k]) * plan->dw_scratch_stride;
-                    b.row[k] = (long long)plan->dw_scratch_stride;
-                }
-            }
-            return b;
-        };
-        std::shared_ptr<gaast::JitKernel> dwk;
-        gaast::DenseMatLaunch mshape;
-        std::shared_ptr<gaast::JitKernel> dmk;
-        if (prog.mat) {
-            mshape = gaast::dense_matrix_shape(*ctx, *prog.mat, n);
-            dmk = dense_matrix_kernel_for(mshape);
-        }
-        for (size_t i = 0; i < prog.steps.size() && dmk; ++i) {
-            const gaast::DenseWarpStep& step = prog.steps[i];
-            cuda_check(gaast::dense_matrix_launch(prog, step, buffers_of(step.L), buffers_of(step.R), buffers_of(step.O),
-                                                  step.C.slot >= 0 ? buffers_of(step.C) : gaast::DenseWarpBuffers(), n,
-                                                  plan->d_dm_src, plan->d_dm_lx, plan->d_dm_rows, mshape,
-                                                  dmk->kernel, ctx->stream),
-                       "launch dense-matrix kernel");
-            ctx->launches += 2;  // the row-address prologue and the product
-        }
-        if (dmk) {
-            grid = mshape.grid;
-            char desc[400];
-            std::snprintf(desc, sizeof desc,
-                          "gaast_dense_matrix engine=dense_warp kernel=matrix origin=%s products=%zu grid=%d block=%d smem=%zu "
-                          "tile=%d elements regs=%d spill=%zuB blocks/SM=%d fma/elem=%d key=%s M%d x%d cols=%d",
-                          dmk->origin.c_str(), prog.steps.size(), grid, mshape.threads, mshape.smem, mshape.T, dmk->regs,
-                          dmk->local_bytes, mshape.blocks_per_sm, dmk->fma_per_elem, dmk->key.c_str(), 1 << prog.mat->mx,
-                          1 << prog.mat->db, 1 << prog.mat->dl);
-            plan->last_kernel = desc;
-        }
-        for (size_t i = 0; i < prog.steps.size() && !dmk; ++i) {
-            const gaast::DenseWarpStep& step = prog.steps[i];
-            dwk = dense_warp_kernel_for(int(i), shape);
-            cuda_check(gaast::dense_warp_launch(prog, step, buffers_of(step.L), buffers_of(step.R), buffers_of(step.O),
-                                                step.C.slot >= 0 ? buffers_of(step.C) : gaast::DenseWarpBuffers(), n,
-                                                plan->d_dw_blades, shape, dwk ? dwk->kernel : nullptr, ctx->stream),
-                       "launch dense-warp engine");
-            ctx->launches++;
-        }
-        if (!dmk) {
-            char desc[320];
-            std::snprintf(desc, sizeof desc,
-                          "%s engine=dense_warp origin=%s products=%zu grid=%d block=%d smem=%zu tile=%d elements regs=%d",
-                          dwk ? "gaast_dense_warp" : "dense_warp_kernel", dwk ? dwk->origin.c_str() : "library",
-                          prog.steps.size(), grid, shape.threads, shape.smem, shape.T, dwk ? dwk->regs : 0);
-            plan->last_kernel = desc;
-        }
-    } else if (jk) {
-        const long long per_block = (long long)jk->threads * jk->elems_per_thread;
-        const long long blocks = (n + per_block - 1) / per_block;
-        if (blocks > 0x7fffffffLL) throw Error(GAAST_ERR_SHAPE, "batch too long for one launch");
-        grid = int(blocks);
-        size_t max_grid = size_t(grid);
-        if ((with_sum || jk->pipelined || gaast::tuning().force_persistent) && !jk->one_tile_blocks) {
-            // persistent grid: the batch-sum epilogue keeps per-block partials, and the TMA-pipelined
-            // kernels loop over their tiles; blocks stride over the batch
-            // sum-only kernels: many short-lived blocks overlap better than one long-lived block per resident slot, but
-            // every block pays its epilogue (column sums -> partials), so a block should still see ~8 tiles.  Measured
-            // on cfg5 + sum (ms per step at 4 / 8 / 16 / 32 / 64 blocks per slot): 32 M elements 6.42 / 6.20 / - / 5.97 /
-            // 5.92; 8 M (the 4-GPU shard) 1.577 / 1.535 / 1.505 / 1.501 / 1.558; 4 M (the 8-GPU shard) 0.787 / 0.770 /
-            // 0.770 / 0.793 / 0.857.
-            const long long resident = (long long)ctx->sm_count * jk->blocks_per_sm;
-            long long mult = jk->pipelined ? 1 : std::min(64LL, std::max(4LL, blocks / (8 * resident)));
-            if (gaast::tuning().grid_mult > 0) mult = gaast::tuning().grid_mult;
-            const long long cap = resident * mult;
-            if (grid > cap) grid = int(cap);
-            max_grid = size_t(resident * std::max(64LL, mult));  // scratch sized once, for the largest grid of the variant
-        }
-        if (with_sum) {
-            // sized for the largest grid this kernel can get: allocated by the first call, never again
-            ensure(plan->d_partials, plan->partials_cap, (std::max(max_grid, size_t(grid)) + gaast::kReduceStage1Rows) * sum_cols);
-            a.partials = plan->d_partials;
-        }
-        if (jk->n_uniform > 0) {
-            ensure(plan->d_uniform, plan->uniform_cap, size_t(jk->n_uniform));
-            a.uniform = plan->d_uniform;
-            void* params[] = {&a};
-            cuda_check(cudaLaunchKernel(reinterpret_cast<const void*>(jk->uniform_kernel), dim3(1), dim3(32), params, 0,
-                                        ctx->stream),
-                       "launch uniform prologue");
-            ctx->launches++;
-        }
-        a.lookahead = ctx->sm_count * jk->blocks_per_sm;  // resident blocks: the look-ahead distance of the L2 prefetch variant
-        if (gaast::tuning().lookahead >= 0) a.lookahead = gaast::tuning().lookahead;
-        void* params[] = {&a};
-        cuda_check(cudaLaunchKernel(reinterpret_cast<const void*>(jk->kernel), dim3(grid), dim3(jk->threads), params, jk->smem_bytes,
-                                    ctx->stream),
-                   "launch specialised kernel");
-        ctx->launches++;
-        char desc[512];
-        std::snprintf(desc, sizeof desc,
-                      "%s engine=specialized origin=%s grid=%d block=%d elems/thread=%d regs=%d spill=%zuB fma/elem=%d key=%s",
-                      jk->name.c_str(), jk->origin.c_str(), grid, jk->threads, jk->elems_per_thread, jk->regs,
-                      jk->local_bytes, jk->fma_per_elem, jk->key.c_str());
-        plan->last_kernel = desc;
-    } else {
-        gaast::TableLaunch shape = gaast::table_engine_shape(*ctx, h, n, with_sum, f32);
-        grid = shape.grid;
-        // scratch is sized for the largest grid the engine ever launches (8 blocks per SM), so that only the
-        // first call allocates
-        const size_t max_grid = std::max(size_t(grid), size_t(ctx->sm_count) * 8);
-        if (shape.global_ws) {
-            ensure(plan->d_ws, plan->ws_cap, max_grid * shape.ws_doubles_per_block);
-            a.ws_global = plan->d_ws;
-        }
-        if (with_sum) {
-            ensure(plan->d_partials, plan->partials_cap, (max_grid + gaast::kReduceStage1Rows) * sum_cols);
-            a.partials = plan->d_partials;
-        }
-        a.micro = plan->d_micro;
-        a.chunks = plan->d_chunks;
-        a.n_micro = int(h.micro.size());
-        a.n_chunks = int(h.chunks.size());
-        cuda_check(gaast::table_engine_launch(a, shape, arith == GAAST_ARITH_STRICT, with_sum, f32, ctx->stream),
-                   "launch table engine");
-        ctx->launches++;
-        char desc[256];
-        std::snprintf(desc, sizeof desc, "table_engine_kernel engine=table grid=%d block=%d smem=%zu ws=%s", grid,
-                      shape.threads, shape.smem, shape.global_ws ? "global" : "shared");
-        plan->last_kernel = desc;
-    }
+    const Engine e = choose_engine(c, engine, &jk);
+    const int grid = e == Engine::dense_warp ? launch_dense_warp(c) : e == Engine::specialized ? launch_specialized(c, *jk)
+                                                                                                : launch_table(c);
     if (with_sum) {
         cuda_check(gaast::reduce_partials_launch(plan->d_partials, grid, sum_cols, dev_sum, ctx->stream),
                    "launch partial-sum reduction");

@@ -54,6 +54,11 @@ struct CodegenOptions {
     // for finite y); stored rows are addressed by their rank.
     std::vector<std::vector<uint64_t>> sparse;
     uint64_t sparse_hash = 0;
+    // What tells two specialised kernels of one plan apart (the bitmaps by their hash): the plan's map key.
+    auto key() const {
+        return std::make_tuple(broadcast_slots, arith, with_sum, store_out, elems_per_thread, variant, pipelined, tma_stage,
+                               f32, sparse_hash);
+    }
 };
 
 struct CodegenResult {
@@ -246,8 +251,8 @@ struct gaast_plan {
     double* d_uniform = nullptr;
     size_t uniform_cap = 0;
     std::string last_kernel;
-    // specialised kernels, keyed by (broadcast slots, arith, with_sum, store_out, elems/thread, variant)
-    using JitKey = std::tuple<uint64_t, int, int, int, int, int, int, int, int, uint64_t>;
+    // specialised kernels, keyed by the options they were generated with
+    using JitKey = decltype(gaast::CodegenOptions().key());
     std::map<JitKey, std::shared_ptr<gaast::JitKernel>> jit;
     // why a variant could not be built (its entry in `jit` is null): per variant, never sticky for the plan
     std::map<JitKey, std::string> jit_errors;

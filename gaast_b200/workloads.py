@@ -210,6 +210,19 @@ def torch_inputs(w: Workload, length: int, device, seed: int = None):
 
 
 # ---- build-time kernel cache --------------------------------------------------------
+def precompile_variants(w: Workload):
+    """The (arith, with_sum, store_out, dtype) calls of `w` whose kernels the build compiles ahead of time."""
+    from . import _lib as L
+    variants = [(L.ARITH_FMA, False, True, L.F64), (L.ARITH_STRICT, False, True, L.F64)]
+    if w.sum_root:
+        variants += [(L.ARITH_FMA, True, True, L.F64), (L.ARITH_FMA, True, False, L.F64)]
+    # the f32 variant of the same plans (bench.py --dtype f32, tests/test_gpu_f32.py)
+    variants += [(L.ARITH_FMA, False, True, L.F32), (L.ARITH_STRICT, False, True, L.F32)]
+    if w.sum_root:
+        variants += [(L.ARITH_FMA, True, True, L.F32)]
+    return variants
+
+
 def precompile_all(verbose: bool = False, fresh: bool = True) -> int:
     """Generate + compile the specialised kernels of every workload (no device needed)."""
     import os
@@ -222,14 +235,7 @@ def precompile_all(verbose: bool = False, fresh: bool = True) -> int:
     count = 0
     for w in WORKLOADS.values():
         plan = Plan(None, specialize(w))
-        variants = [(L.ARITH_FMA, False, True, L.F64), (L.ARITH_STRICT, False, True, L.F64)]
-        if w.sum_root:
-            variants += [(L.ARITH_FMA, True, True, L.F64), (L.ARITH_FMA, True, False, L.F64)]
-        # the f32 variant of the same plans (bench.py --dtype f32, tests/test_gpu_f32.py)
-        variants += [(L.ARITH_FMA, False, True, L.F32), (L.ARITH_STRICT, False, True, L.F32)]
-        if w.sum_root:
-            variants += [(L.ARITH_FMA, True, True, L.F32)]
-        for arith, with_sum, store, dtype in variants:
+        for arith, with_sum, store, dtype in precompile_variants(w):
             info = plan.precompile(w.broadcast_mask(), arith, with_sum, store, dtype)
             count += 1
             if verbose:

@@ -213,16 +213,20 @@ FAULTS = {1: "a barrier / shuffle in sequential mode", 2: "a bulk copy that is n
 def run_generated_kernel(ast, inputs: Sequence[Dict[int, np.ndarray]], broadcast: Sequence[bool], batch: int,
                          arith: int = L.ARITH_FMA, with_sum: bool = False, tuning: Optional[Tuple[int, int]] = None,
                          grid: Optional[int] = None, store_out: bool = True, dtype=np.float64,
-                         present: Optional[Dict] = None):
+                         present: Optional[Dict] = None, components: Optional[Dict[int, Sequence[int]]] = None):
     """Evaluate the specialised engine's kernel for `ast` (a gaast_b200.expr.SpecializedAst) on host arrays.
     inputs[slot] = {grade: (C(n,k), batch) array, or (C(n,k), 1) for a broadcast slot}.
     present = {(slot, grade): stored component indices} for inputs in sparse per-grade storage: that grade's array
     then holds the stored rows only, in component order.
+    components = {root grade: stored component indices} makes the plan a projected one (gaast_plan_create_projected; a
+    grade that is not listed is kept whole): out[k] and sums[k] then hold the stored components of grade k only, in
+    component order.
     Returns (out: {grade: (C, batch)}, sums or None, info) where info = {"notes", "threads", "ept", "grid", "source"}."""
-    plan = g.Plan(None, ast)
+    plan = g.Plan(None, ast, components=components)
     if tuning is not None:
         plan.set_tuning(*tuning)
     n = plan.n
+    root_rows = {k: len(set(components[k])) if components and k in components else comb(n, k) for k in plan.root_grades()}
     slots = plan.num_slots()
     bmask = sum(1 << s for s in range(slots) if broadcast[s])
     f32 = dtype == np.float32
@@ -255,7 +259,7 @@ def run_generated_kernel(ast, inputs: Sequence[Dict[int, np.ndarray]], broadcast
             si += 1
     outs = {}
     for k in plan.root_grades():
-        arr = np.full((comb(n, k), padded), np.nan, dtype=dtype)
+        arr = np.full((max(1, root_rows[k]), padded), np.nan, dtype=dtype)[:root_rows[k]]  # (an emptied grade: no rows)
         outs[k] = arr
         launch.sptr[si] = arr.ctypes.data
         launch.srow[si] = padded
@@ -264,7 +268,7 @@ def run_generated_kernel(ast, inputs: Sequence[Dict[int, np.ndarray]], broadcast
     desc = ast.lower().contents
     consts = np.array([desc.const_values[i] for i in range(desc.n_const_values)] + [0.0], dtype=np.float64)
     uniform = np.full(1 << 16, np.nan)
-    root_cols = sum(comb(n, k) for k in plan.root_grades())
+    root_cols = sum(root_rows.values())
     threaded = needs_threads(src)
     if grid is None:
         grid = max(1, (batch + per_block - 1) // per_block)
@@ -297,8 +301,8 @@ def run_generated_kernel(ast, inputs: Sequence[Dict[int, np.ndarray]], broadcast
         sums, c = {}, 0
         tot = partials[:grid].sum(axis=0)
         for k in plan.root_grades():
-            sums[k] = tot[c:c + comb(n, k)]
-            c += comb(n, k)
+            sums[k] = tot[c:c + root_rows[k]]
+            c += root_rows[k]
     info = {"notes": src.split("\n")[1], "threads": threads, "ept": ept, "grid": grid, "threaded": threaded,
             "source": src}
     return out, sums, info

@@ -84,6 +84,30 @@ def test_generated_kernels_compile_for_sm100a(scratch_cache):
     assert "origin=override" in info2 and "unverified" not in info2  # a redirected cache says so in the origin
 
 
+def test_kernel_source_is_the_precompiled_kernel(scratch_cache):
+    """gaast_plan_kernel_source returns the text of the kernel gaast_plan_precompile compiles (the one gaast_eval
+    launches for an aligned batch), for every call of every workload whose kernel the build precompiles.  It runs in a
+    fresh process, as the build does: once torch is imported, NVRTC is torch's, whose ptxas may report spills, and a
+    kernel that spills is rebuilt with more rows parked in shared memory."""
+    import subprocess
+    import sys
+    check = """if True:
+        import os
+        import gaast_b200 as g
+        from gaast_b200 import workloads as W
+        for w in W.WORKLOADS.values():
+            plan = g.Plan(None, W.specialize(w))
+            for arith, with_sum, store_out, dtype in W.precompile_variants(w):
+                kw = dict(broadcast_slots=w.broadcast_mask(), arith=arith, with_sum=with_sum, store_out=store_out, dtype=dtype)
+                key = [t for t in plan.precompile(**kw).split() if t.startswith("key=")][0][4:]
+                src = open(os.path.join(os.environ["GAAST_KERNEL_CACHE"], key + ".cu")).read()
+                assert src == plan.kernel_source(**kw), (w.name, kw)
+            plan.free()
+    """
+    r = subprocess.run([sys.executable, "-c", check], cwd=ROOT, capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-3000:]
+
+
 def test_kernel_cache_override_needs_the_test_hook(tmp_path, monkeypatch):
     """GAAST_KERNEL_CACHE alone does not redirect the cache: the in-tree one keeps serving."""
     monkeypatch.setenv("GAAST_KERNEL_CACHE", str(tmp_path))

@@ -1,6 +1,5 @@
 """Projected plans (gaast_plan_create_projected) on a machine without a GPU: the kernel text of an offline plan, and the
-generated kernels executed by the CPU stand-in of tests/kernel_emu (through tests/projection_emu.py) against the
-oracle's selected rows.
+generated kernels executed by the CPU stand-in of tests/kernel_emu against the oracle's selected rows.
 
 A projected plan keeps only chosen root components; the others are zero and are neither computed nor stored.  In
 strict arithmetic every stored component is bit-identical to the oracle (each output keeps the reference's term order),
@@ -15,7 +14,7 @@ import gaast_b200 as g
 from gaast_b200 import _lib as L
 from gaast_b200 import workloads as W
 from tests.helpers import REL_TOL_F32, assert_bit_exact, assert_close, oracle_abs_scale, oracle_eval, run_plan_numpy
-from tests.projection_emu import run_projected_kernel
+from tests.kernel_emu import run_generated_kernel
 
 pytestmark = pytest.mark.timeout(600)
 
@@ -69,10 +68,10 @@ def test_projected_kernels_match_oracle(name):
     bcs = [bc for _, bc in w.inputs]
     want = select(oracle_eval(w.build, w.metric, host, bcs, batch), comps)
     scale = select(oracle_abs_scale(w.build, w.metric, host, bcs, batch), comps)
-    out, _, info = run_projected_kernel(ast, host, bcs, batch, arith=L.ARITH_STRICT, components=comps)
+    out, _, info = run_generated_kernel(ast, host, bcs, batch, arith=L.ARITH_STRICT, components=comps)
     assert "projection(" in info["notes"], info["notes"]
     assert_bit_exact(out, want, f"{name} projected strict [{info['notes']}]")
-    out, _, info = run_projected_kernel(ast, host, bcs, batch, arith=L.ARITH_FMA, components=comps)
+    out, _, info = run_generated_kernel(ast, host, bcs, batch, arith=L.ARITH_FMA, components=comps)
     assert_close(out, want, scale, what=f"{name} projected fma [{info['notes']}]")
 
 
@@ -87,9 +86,9 @@ def test_projected_kernels_f32(name):
     bcs = [bc for _, bc in w.inputs]
     with np.errstate(all="ignore"):
         want32 = select(run_plan_numpy(ast.plan_dict(), host, batch, dtype=np.float32), comps)
-    out, _, info = run_projected_kernel(ast, host, bcs, batch, arith=L.ARITH_STRICT, dtype=np.float32, components=comps)
+    out, _, info = run_generated_kernel(ast, host, bcs, batch, arith=L.ARITH_STRICT, dtype=np.float32, components=comps)
     assert_bit_exact(out, want32, f"{name} projected f32 strict [{info['notes']}]")
-    out, _, info = run_projected_kernel(ast, host, bcs, batch, arith=L.ARITH_FMA, dtype=np.float32, components=comps)
+    out, _, info = run_generated_kernel(ast, host, bcs, batch, arith=L.ARITH_FMA, dtype=np.float32, components=comps)
     want = select(oracle_eval(w.build, w.metric, host64, bcs, batch), comps)
     scale = select(oracle_abs_scale(w.build, w.metric, host64, bcs, batch), comps)
     assert_close({k: v.astype(np.float64) for k, v in out.items()}, want, scale, rel=REL_TOL_F32,
@@ -113,7 +112,7 @@ def test_projected_batch_sum(name, variant, store_out):
     bcs = [bc for _, bc in w.inputs]
     want = select(oracle_eval(w.build, w.metric, host, bcs, batch), comps)
     scale = select(oracle_abs_scale(w.build, w.metric, host, bcs, batch), comps)
-    out, sums, info = run_projected_kernel(ast, host, bcs, batch, arith=L.ARITH_FMA, with_sum=True, store_out=store_out,
+    out, sums, info = run_generated_kernel(ast, host, bcs, batch, arith=L.ARITH_FMA, with_sum=True, store_out=store_out,
                                            tuning=(0, variant), grid=2, components=comps)
     if variant & 262144:
         assert "sum-in-tmem" in info["notes"], info["notes"]
@@ -137,7 +136,7 @@ def test_projected_plan_with_sparse_inputs():
     want = oracle_eval(w.build, w.metric, host, [False, False], batch)
     comps = {2: [0, 5, 11, 17, 30, 41, 52, 60, 65]}
     sparse_host = [host[0], {2: host[1][2][keep_in]}]
-    out, _, info = run_projected_kernel(ast, sparse_host, [False, False], batch, arith=L.ARITH_STRICT,
+    out, _, info = run_generated_kernel(ast, sparse_host, [False, False], batch, arith=L.ARITH_STRICT,
                                         present={(1, 2): keep_in}, components=comps)
     assert_bit_exact(out, select(want, comps), f"sparse inputs + projection [{info['notes']}]")
 
