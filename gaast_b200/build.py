@@ -37,6 +37,7 @@ SOURCES = [
     "device/dense_warp.cu",
     "device/dense_matrix.cu",
     "device/records.cu",
+    "device/segments.cu",
     "device/runtime.cu",
     "device/host_pipeline.cu",
     "device/diag.cu",

@@ -609,10 +609,11 @@ int gaast_batch_dtype(const gaast_batch* b) { return b ? b->dtype : GAAST_F64; }
 gaast_status gaast_batch_free(gaast_batch* b) {
     return guard([&] {
         if (!b) return;
-        if ((b->owned && b->base) || !b->records.empty()) {
+        if ((b->owned && b->base) || !b->records.empty() || b->segment_scratch) {
             DeviceGuard dg(b->ctx->device);
             if (b->owned && b->base) cudaFree(b->base);
             for (auto& kv : b->records) cudaFree(kv.second.d_table);
+            if (b->segment_scratch) cudaFree(b->segment_scratch);
         }
         delete b;
     });
@@ -671,6 +672,8 @@ gaast_status gaast_batch_zero(gaast_batch* b) {
 }
 
 // ------------------------------------------------------------- records ----
+static const gaast::RecordMap& record_map(const gaast_batch* b, uint32_t record_mask);
+
 // Checks a records call and returns the batch's row map for `record_mask`, building it on the first call (null when
 // count == 0: nothing to do).
 static const gaast::RecordMap* records_prepare(const gaast_batch* b, uint64_t first, uint64_t count, uint32_t record_mask,
@@ -684,8 +687,13 @@ static const gaast::RecordMap* records_prepare(const gaast_batch* b, uint64_t fi
     if (first > b->len || count > b->len - first)
         throw Error(GAAST_ERR_SHAPE, std::string(what) + ": first + count exceeds the batch length");
     if (!count) return nullptr;
+    return &record_map(b, record_mask);
+}
+
+// The batch's row map for `record_mask` (a superset of its grades), built on the first request.
+static const gaast::RecordMap& record_map(const gaast_batch* b, uint32_t record_mask) {
     auto it = b->records.find(record_mask);
-    if (it != b->records.end()) return &it->second;
+    if (it != b->records.end()) return it->second;
     // stored rows in record-component order: grades ascending, within a grade the stored components ascending
     std::vector<gaast::RecordRow> rows;
     const size_t es = b->esize();
@@ -723,7 +731,7 @@ static const gaast::RecordMap* records_prepare(const gaast_batch* b, uint64_t fi
         cudaFree(m.d_table);
         cuda_check(e, "upload record row map");
     }
-    return &b->records.emplace(record_mask, m).first->second;
+    return b->records.emplace(record_mask, m).first->second;
 }
 
 // Device entry points: `records` must be device memory the kernel can address, aligned to the scalar type.
@@ -802,6 +810,50 @@ gaast_status gaast_batch_upload_records(gaast_batch* b, uint64_t first, uint64_t
 gaast_status gaast_batch_download_records(const gaast_batch* b, uint64_t first, uint64_t count, void* host_records,
                                           uint32_t record_mask) {
     return guard([&] { records_host(b, first, count, host_records, record_mask, true); });
+}
+
+// ------------------------------------------------------------ segments ----
+// `p` must be device or managed memory of the batch's device.
+static void check_device_pointer(const gaast_batch* b, const void* p, const char* what) {
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, p) != cudaSuccess) {
+        cudaGetLastError();
+        throw Error(GAAST_ERR_INVALID, std::string("segment_sum: ") + what + " is not known to CUDA");
+    }
+    const bool ok = attr.type == cudaMemoryTypeManaged || (attr.type == cudaMemoryTypeDevice && attr.device == b->ctx->device);
+    if (!ok) throw Error(GAAST_ERR_INVALID, std::string("segment_sum: ") + what + " is not device memory of the batch's device");
+}
+
+gaast_status gaast_batch_segment_sum(const gaast_batch* b, const int64_t* dev_offsets, uint64_t n_segments, double* dev_sums) {
+    return guard([&] {
+        if (!b) throw Error(GAAST_ERR_INVALID, "segment_sum: null batch");
+        if (b->broadcast) throw Error(GAAST_ERR_SHAPE, "segment_sum: a broadcast batch has no segments");
+        if (!n_segments) return;
+        if (!dev_offsets || !dev_sums) throw Error(GAAST_ERR_INVALID, "segment_sum: null offsets or sums pointer");
+        if (reinterpret_cast<uintptr_t>(dev_offsets) % 8 || reinterpret_cast<uintptr_t>(dev_sums) % 8)
+            throw Error(GAAST_ERR_INVALID, "segment_sum: offsets and sums must be 8-byte aligned");
+        DeviceGuard dg(b->ctx->device);
+        check_device_pointer(b, dev_offsets, "the offsets pointer");
+        check_device_pointer(b, dev_sums, "the sums pointer");
+        if (!b->rows) return;  // (no stored row: nothing to write)
+        const gaast::RecordMap& m = record_map(b, b->mask);  // stored rows in the order of the sums
+        gaast_ctx* ctx = b->ctx;
+        if (!b->segment_scratch) {
+            const size_t bytes = gaast::segment_scratch_bytes((long long)b->len, int(b->rows));
+            cuda_check(cudaMalloc(&b->segment_scratch, bytes), "cudaMalloc(segment-sum partials)");
+            const cudaError_t e = cudaMemsetAsync(b->segment_scratch, 0, bytes, ctx->stream);
+            if (e != cudaSuccess) {
+                cudaFree(b->segment_scratch);
+                b->segment_scratch = nullptr;
+                cuda_check(e, "clear segment-sum partials");
+            }
+        }
+        cuda_check(gaast::segment_sum_launch(reinterpret_cast<const gaast::RecordRow*>(m.d_table), int(b->rows), b->esize(),
+                                             (long long)b->len, reinterpret_cast<const long long*>(dev_offsets),
+                                             (long long)n_segments, dev_sums, b->segment_scratch, ctx->stream),
+                   "launch gaast_segment_pieces / gaast_segment_spans");
+        ctx->launches += 2;
+    });
 }
 
 // ---------------------------------------------------------------- eval ----

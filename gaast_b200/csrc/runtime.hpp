@@ -205,6 +205,14 @@ void records_shape(RecordMap& m, int K, size_t es, int sm_count);
 cudaError_t records_launch(const RecordMap& m, bool unpack, size_t es, void* records, long long first, long long count,
                            cudaStream_t stream);
 
+// segments.cu: per-segment sums of a batch's stored rows (gaast_batch_segment_sum).  The scratch -- a flag, the chunks'
+// spanning segments and their head / tail partials -- is sized from the batch's length and stored rows and owned by the
+// batch; it must start zeroed.  Two kernel launches.
+size_t segment_scratch_bytes(long long len, int S);
+cudaError_t segment_sum_launch(const RecordRow* rows, int S, size_t es, long long len, const long long* offsets,
+                               long long n, double* sums, void* scratch, cudaStream_t stream);
+long long segment_chunk();  // columns per chunk: fixes the order of the additions
+
 }  // namespace gaast
 
 struct gaast_ctx {
@@ -236,6 +244,7 @@ struct gaast_batch {
     uint32_t stored[GAAST_MAX_DIM + 1] = {};  // rows stored per grade
     bool sparse = false;
     mutable std::map<uint32_t, gaast::RecordMap> records;  // by record mask (gaast_batch_pack_records / _unpack_records)
+    mutable void* segment_scratch = nullptr;  // gaast_batch_segment_sum: allocated on its first call
 };
 
 struct gaast_plan {

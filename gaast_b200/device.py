@@ -236,6 +236,22 @@ class DeviceBatch:
         L.check(L.lib.gaast_batch_unpack_records(self._h, 0, self.length, L.vp(out.data_ptr()), mask))
         return out
 
+    def segment_sum(self, offsets, out=None):
+        """Per-segment sums of the stored rows (gaast_batch_segment_sum): segment j is columns [offsets[j], offsets[j+1]).
+        `offsets` is a CUDA int64 tensor of n_segments + 1 values on the batch's device.  Returns, or fills, a CUDA
+        float64 tensor [n_segments, S] (S = the stored rows, grades ascending); stream-ordered on the ctx stream.
+        Offsets that are not non-decreasing within [0, length] give NaN everywhere."""
+        import torch
+        assert offsets.is_cuda and offsets.dtype == torch.int64 and offsets.dim() == 1 and offsets.is_contiguous(), \
+            "offsets must be a contiguous 1-D CUDA int64 tensor"
+        n_seg = max(0, offsets.shape[0] - 1)
+        S = sum(self.stored_rows(k) for k in self.grade_set())
+        if out is None:
+            out = torch.empty((n_seg, S), dtype=torch.float64, device=offsets.device)
+        assert out.is_cuda and out.dtype == torch.float64 and out.is_contiguous() and tuple(out.shape) == (n_seg, S)
+        L.check(L.lib.gaast_batch_segment_sum(self._h, L.vp(offsets.data_ptr()), n_seg, L.vp(out.data_ptr())))
+        return out
+
     def stored_rows(self, k: int) -> int:
         return L.lib.gaast_batch_stored_rows(self._h, k)
 

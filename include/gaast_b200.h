@@ -336,6 +336,31 @@ gaast_status gaast_batch_upload_records(gaast_batch* b, uint64_t first, uint64_t
 gaast_status gaast_batch_download_records(const gaast_batch* b, uint64_t first, uint64_t count, void* host_records,
                                           uint32_t record_mask);
 
+/* Per-segment sums of a batch's stored rows.  Segment j is batch columns [offsets[j], offsets[j+1]);
+ * dev_sums[j * S + r] = sum over the segment of stored row r (S = the batch's stored rows, over all grades:
+ * grades ascending, stored components ascending -- the order of gaast_eval_sum's vector).  f64 accumulation
+ * for f64 and f32 batches.  offsets: n_segments + 1 int64 values in device memory of the batch's device.
+ *   - Offsets must be non-decreasing with 0 <= offsets[0] and offsets[n_segments] <= len; columns outside
+ *     [offsets[0], offsets[n_segments]) are ignored.  They are read on the device only (checking them on the host
+ *     would need a synchronise), and the kernels stay in bounds whatever their values: offsets that break the rule
+ *     make every one of the n_segments x S doubles NaN -- a documented result, not a fault.
+ *   - Every output double is written (overwritten, not added to); an empty segment gives +0.0.  n_segments == 0
+ *     returns GAAST_OK and launches nothing, and so does a batch that stores no row.
+ *   - Deterministic: the order of the additions depends only on the offsets, the batch length and a chunk size
+ *     compiled into the library (4096 columns), not on the grid or the SM count.  Within a chunk, lane l of 32 adds
+ *     the segment's columns c with c % 32 == l in ascending order from +0.0, and the 32 lane sums are added in an
+ *     aligned binary tree; the pieces of a segment that spans chunks are added in a pairwise tree over the chunks
+ *     (DESIGN.md 3.7).  Repeated calls, CUDA-graph replay and another ctx give bit-identical sums.
+ *   - GAAST_ERR_INVALID: a null batch; a null dev_offsets or dev_sums with n_segments > 0; either pointer not 8-byte
+ *     aligned, or not device (or managed) memory of the batch's device.  GAAST_ERR_SHAPE: a broadcast batch.  These
+ *     checks happen before any launch.
+ *   - Dense and sparse batches (the stored rows only), wrapped ones with stride > len, f64 or f32.
+ *   - Stream-ordered on the ctx stream.  The first call on a batch allocates its scratch (the chunks' partial sums,
+ *     sized from len and S, freed with the batch) and builds the batch's row map; every later call only enqueues two
+ *     kernels (gaast_ctx_launch_count grows by 2) and can be captured in a CUDA graph. */
+gaast_status gaast_batch_segment_sum(const gaast_batch* b, const int64_t* dev_offsets, uint64_t n_segments,
+                                     double* dev_sums);
+
 /* eval: out[i] = expr(inputs[0][i], inputs[1][i], ...) for i in [0, len).
  * `inputs` has plan.n_slots entries; `out` must carry exactly the plan's root
  * grade set (SURVEY.md Q3).  Stream-ordered, asynchronous. */

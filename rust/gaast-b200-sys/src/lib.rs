@@ -111,6 +111,9 @@ pub enum gaast_plan {}
 pub enum gaast_batch {}
 pub enum gaast_comm {}
 
+/// `int64_t` of the header (the CSR offsets of gaast_batch_segment_sum).
+pub type int64_t = i64;
+
 #[link(name = "gaast_b200")]
 extern "C" {
     pub fn gaast_last_error() -> *const c_char;
@@ -163,6 +166,7 @@ extern "C" {
     pub fn gaast_batch_unpack_records(b: *const gaast_batch, first: u64, count: u64, records: *mut c_void, record_mask: u32) -> c_int;
     pub fn gaast_batch_upload_records(b: *mut gaast_batch, first: u64, count: u64, host_records: *const c_void, record_mask: u32) -> c_int;
     pub fn gaast_batch_download_records(b: *const gaast_batch, first: u64, count: u64, host_records: *mut c_void, record_mask: u32) -> c_int;
+    pub fn gaast_batch_segment_sum(b: *const gaast_batch, dev_offsets: *const int64_t, n_segments: u64, dev_sums: *mut f64) -> c_int;
 
     pub fn gaast_eval(plan: *mut gaast_plan, inputs: *const *mut gaast_batch, n_inputs: u32, out: *mut gaast_batch, engine: c_int, arith: c_int) -> c_int;
     pub fn gaast_eval_sum(plan: *mut gaast_plan, inputs: *const *mut gaast_batch, n_inputs: u32, out: *mut gaast_batch, dev_sum: *mut f64, engine: c_int, arith: c_int) -> c_int;
