@@ -100,19 +100,22 @@ class DeviceBatch:
 
     @staticmethod
     def wrap_torch(ctx: Ctx, n: int, tensors: Dict[int, "object"], broadcast: bool = False) -> "DeviceBatch":
-        """Wrap caller-owned CUDA float64 (or, all of them, float32) tensors {grade: [C(n,k), len]} (row-major)."""
+        """Wrap caller-owned CUDA float64 (or, all of them, float32) tensors {grade: [C(n,k), len]} (row-major).  The
+        batch's row stride is that of its multi-row tensors (a one-row grade has none of its own)."""
         grades = sorted(tensors)
-        length, stride = None, None
+        length = None
         ptrs = []
         kinds = {str(t.dtype) for t in tensors.values()}
         assert kinds <= {"torch.float64"} or kinds <= {"torch.float32"}, "one scalar type per batch"
         dtype = L.F32 if kinds == {"torch.float32"} else L.F64
+        multi = [tensors[k] for k in grades if tensors[k].shape[0] > 1]
+        stride = multi[0].stride(0) if multi else (tensors[grades[0]].shape[1] if grades else 0)
         for k in grades:
             t = tensors[k]
             assert t.is_cuda and t.dim() == 2 and t.shape[0] == comb(n, k)
             assert t.stride(1) == 1 or t.shape[1] == 1
             if length is None:
-                length, stride = t.shape[1], (t.stride(0) if t.shape[0] > 1 else t.shape[1])
+                length = t.shape[1]
             assert t.shape[1] == length
             if t.shape[0] > 1:
                 assert t.stride(0) == stride, "all grades must share one row stride"

@@ -24,6 +24,7 @@ import numpy as np
 
 import gaast_b200 as g
 from gaast_b200 import _lib as L
+from tests.guarded_layout import BITS, poison, sentinel
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 MAX_STREAMS = 96
@@ -245,13 +246,14 @@ def run_generated_kernel(ast, inputs: Sequence[Dict[int, np.ndarray]], broadcast
         for k in plan.slot_grades(s):
             rows = len(present[(s, k)]) if present and (s, k) in present else comb(n, k)
             src_arr = np.asarray(inputs[s][k], dtype=dtype)
+            # the padding holds the input sentinel: it is never part of a result
             if broadcast[s]:
-                arr = np.zeros((rows, 4), dtype=dtype)
+                arr = poison(np.empty((rows, 4), dtype=dtype), "in")
                 arr[:, 0] = src_arr.reshape(rows, -1)[:, 0]
                 launch.bcast[si >> 6] |= 1 << (si & 63)
             else:
                 assert src_arr.shape == (rows, batch), (src_arr.shape, rows, batch)
-                arr = np.full((rows, padded), np.nan, dtype=dtype)  # the padding is never part of a result
+                arr = poison(np.empty((rows, padded), dtype=dtype), "in")
                 arr[:, :batch] = src_arr
             keep.append(arr)
             launch.sptr[si] = arr.ctypes.data
@@ -259,7 +261,7 @@ def run_generated_kernel(ast, inputs: Sequence[Dict[int, np.ndarray]], broadcast
             si += 1
     outs = {}
     for k in plan.root_grades():
-        arr = np.full((max(1, root_rows[k]), padded), np.nan, dtype=dtype)[:root_rows[k]]  # (an emptied grade: no rows)
+        arr = poison(np.empty((max(1, root_rows[k]), padded), dtype=dtype), "out")[:root_rows[k]]  # (an emptied grade: no rows)
         outs[k] = arr
         launch.sptr[si] = arr.ctypes.data
         launch.srow[si] = padded
@@ -295,6 +297,11 @@ def run_generated_kernel(ast, inputs: Sequence[Dict[int, np.ndarray]], broadcast
     launch.which = 0
     rc = lib.emu_launch(C.byref(launch))
     assert rc == 0, f"generated kernel: {FAULTS.get(rc, rc)}"
+    # write containment: the aligned kernel may store into the padding columns it was launched over, and nowhere else
+    for k, v in outs.items():
+        stray = np.argwhere(v[:, launch_n:].view(BITS[v.dtype]) != sentinel(v.dtype, "out"))
+        assert not len(stray), (f"generated kernel: {len(stray)} store(s) beyond the launch length {launch_n}; first: grade "
+                                f"{k} row {stray[0][0]} column {launch_n + stray[0][1]}")
     out = {k: v[:, :batch].copy() for k, v in outs.items()}
     sums = None
     if with_sum:
