@@ -29,6 +29,7 @@ ENGINE_AUTO, ENGINE_TABLE, ENGINE_SPECIALIZED, ENGINE_DENSE_WARP = 0, 1, 2, 3
 HOST_DEFAULT, HOST_WRITE_COMBINED = 0, 1
 COMM_AUTO, COMM_NCCL, COMM_PEER = 0, 1, 2
 ARITH_FMA, ARITH_STRICT = 0, 1
+ARITH_F64 = 2  # a flag OR-ed into either: f32 batches evaluated in binary64, one rounding per stored result
 F64, F32 = 0, 1  # gaast_dtype
 
 OP_ADD_INPUT, OP_MUL_TERMS, OP_NEG_GRADES, OP_SCALAR_INV, OP_SCALAR_SQRT, OP_EXP, OP_LOG = range(7)

@@ -93,12 +93,17 @@ struct Gen {
 
     // Scalar type of the generated arithmetic: "double", or "float" for the f32 variant.  Every
     // emitted declaration goes through it, so the f64 text is unchanged by the f32 support.
+    // Shared-memory values (parked rows, the sums) are of that type too; the batches' own type is f32_store's:
+    // f32 batches evaluated in binary64 (opt.wide) load binary32, compute, park and sum binary64, and round
+    // each stored result once.
     const bool f32;
+    const bool f32_store;
     const std::string S;
     const size_t esize;
 
     Gen(const DevicePlanHost& hh, const CodegenOptions& o)
-        : h(hh), opt(o), strict(o.arith == GAAST_ARITH_STRICT), f32(o.f32), S(o.f32 ? "float" : "double"), esize(o.f32 ? 4 : 8) {}
+        : h(hh), opt(o), strict(o.arith == GAAST_ARITH_STRICT), f32(o.f32 && !o.wide), f32_store(o.f32),
+          S(o.f32 && !o.wide ? "float" : "double"), esize(o.f32 && !o.wide ? 4 : 8) {}
 
     // A projected plan stores root column `col` only when root_row[col] >= 0.  With `prune`, root liveness starts from
     // those columns alone (set after the lowering passes, which match patterns on the whole root buffer).
@@ -1569,7 +1574,7 @@ struct Gen {
         file_scope << "};\n";
         // ---- per-block table of output offsets (the root's grade arrays are separate allocations) ----
         kernel_setup << "  long long* const dense_out = reinterpret_cast<long long*>(sums);\n";
-        if (f32)  // EvalArgs carries the array addresses as double*: measure the distance in floats
+        if (f32_store)  // EvalArgs carries the array addresses as double*: measure the distance in floats
             kernel_setup << "  if (tid < " << B << ")\n    dense_out[tid] = (long long)(reinterpret_cast<const float*>(a.sptr[kDenseOutStream[tid]]) - "
                          << "reinterpret_cast<const float*>(a.sptr[" << root0
                          << "])) + (long long)kDenseOutRow[tid] * a.srow[kDenseOutStream[tid]];\n  __syncthreads();\n";
@@ -1679,7 +1684,7 @@ struct Gen {
             // (with the operand in tensor memory whole warps run: a lane past the end of the batch shadows the last
             // element and must not store -- unguarded, its result from a stale staging row overwrote that element)
             if (guard_stores) line("if (active) {");
-            line(S + "* const ro = s" + std::to_string(root0) + " + e;");
+            line(std::string(f32_store ? "float" : "double") + "* const ro = s" + std::to_string(root0) + " + e;");
             for (int ol = 0; ol < 16; ++ol)
                 line("ro[dense_out[(oh << " + std::to_string(hb) + ") + " +
                      std::to_string(ol) + "]] = q" + std::to_string(ol) + ";");
@@ -1965,6 +1970,22 @@ __device__ __forceinline__ float d_exps(float a) { return (float)s_exps(a); }
 __device__ __forceinline__ float d_logf(float a, float q) { return (float)s_logf(a, q); }
 )GAAST";
 
+// f32 batches evaluated in binary64 (GAAST_ARITH_F64): the f64 prelude above, plus loads of binary32 rows that widen
+// and stores into them that round once, to nearest even.  Parked rows and sums hold the binary64 values.
+const char kPreludeWide[] = R"GAAST(#if GAAST_EPT == 2
+__device__ __forceinline__ D d_load(const float* p) {
+  const float2 v = __ldg(reinterpret_cast<const float2*>(p));
+  return make_double2(v.x, v.y);
+}
+__device__ __forceinline__ void d_store(float* p, D v) {
+  *reinterpret_cast<float2*>(p) = make_float2(__double2float_rn(v.x), __double2float_rn(v.y));
+}
+#else
+__device__ __forceinline__ D d_load(const float* p) { return (double)__ldg(p); }
+__device__ __forceinline__ void d_store(float* p, D v) { *p = __double2float_rn(v); }
+#endif
+)GAAST";
+
 }  // namespace
 
 static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt, bool prune) {
@@ -2028,14 +2049,16 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
     for (const Node& n : g.nodes)
         if (n.live && n.k == N_LOAD && !n.uniform) ++live_loads;
     const size_t root_cols = h.stored_cols;  // batch-sum columns
-    // (an f32 value takes one register instead of two: the budgets below nearly double)
-    const size_t kAccBudget = opt.f32 ? 128 : 72;  // values a thread can keep as accumulators next to its operands
+    // (an f32 value takes one register instead of two: the budgets below nearly double.  f32 batches evaluated in
+    // binary64 hold f64 values: the f64 budgets)
+    const bool cf32 = g.f32;
+    const size_t kAccBudget = cf32 ? 128 : 72;  // values a thread can keep as accumulators next to its operands
     g.op_policy.assign(h.ops.size() + 1, P_TABLE);
     size_t widest = 0;
     int res_parked = 0, res_parkable = 0;
     size_t live_estimate = 0;  // doubles a thread keeps live (widest in-register product + resident rows)
-    const size_t kDenseBudget = opt.f32 ? 160 : 110;  // values: outputs + operands of a product that may all be live
-    const size_t kLiveBudget = opt.f32 ? 224 : 124;   // values a thread can hold in 255 registers next to addresses
+    const size_t kDenseBudget = cf32 ? 160 : 110;  // values: outputs + operands of a product that may all be live
+    const size_t kLiveBudget = cf32 ? 224 : 124;   // values a thread can hold in 255 registers next to addresses
     std::vector<int> uses(g.nodes.size(), 0);  // how many live product terms read each node
     std::set<int> blocked_loads;
     size_t widest_table = 0;
@@ -2073,7 +2096,7 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
             size_t row_opnds = 0;
             for (int id : ls) row_opnds += rowish(id);
             for (int id : rs) row_opnds += rowish(id);
-            if (outs.size() + row_opnds > kLiveBudget + (opt.f32 ? 64 : 32)) pol = P_GATHER;
+            if (outs.size() + row_opnds > kLiveBudget + (cf32 ? 64 : 32)) pol = P_GATHER;
         }
         if (dense && outs.size() <= 144) pol = P_BLOCKED;  // (up to 2 x the f64 accumulator budget)
         if (opt.variant & 1) pol = P_TABLE;
@@ -2162,7 +2185,7 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
         }
     }
     int ept = opt.elems_per_thread;
-    if (ept != 1 && ept != 2) ept = (live_loads + root_cols + widest <= (opt.f32 ? 96u : 48u)) ? 2 : 1;
+    if (ept != 1 && ept != 2) ept = (live_loads + root_cols + widest <= (cf32 ? 96u : 48u)) ? 2 : 1;
     if (n_smem_rows) ept = 1;  // the staging area holds one double per row and thread
     g.ept = ept;
     const int threads = (opt.variant & 16384) ? 64 : 128;  // (tuning knob: 64-thread blocks = twice as many, half as large tiles per SM)
@@ -2203,7 +2226,8 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
     // with a few dozen parked rows next to register rows, LDG + STS is as fast (cfg5: 0.83 vs 0.80)
     bool has_dense = false;
     for (Policy p : g.op_policy) has_dense |= p == P_DENSE || p == P_BLOCKED;
-    const bool tma_stage = opt.tma_stage && has_dense && n_smem_rows > 0 && ept == 1 && !pipelined && !opt.with_sum;
+    // (f32 batches evaluated in binary64 park the widened values: binary32 rows cannot be copied in as they are)
+    const bool tma_stage = opt.tma_stage && has_dense && n_smem_rows > 0 && ept == 1 && !pipelined && !opt.with_sum && !opt.wide;
     const bool par_issue = (opt.variant & 256) && !opt.f32;     // opt-in experiments (f64 only), see DESIGN.md
     const bool look_ahead = (opt.variant & 32768) && !opt.f32;
     g.dense_tmem = tma_stage && g.dense.op >= 0 && (opt.variant & 8192) && !opt.f32;
@@ -2215,6 +2239,7 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
     res.pipelined = pipelined;
     res.smem_bytes = pipelined ? pipe_bytes : sum_doubles * 8 + size_t(n_smem_rows) * threads * g.esize + (tma_stage ? 16 : 0);
     res.one_tile_blocks = tma_stage;
+    if (opt.wide) notes << "f32-storage-f64-arith(f64 staging, no tma) ";
     if (tma_stage) notes << "tma-staged ";
     if (tmem_sum) notes << "sum-in-tmem(" << tmem_cols << "cols,stash=" << g.sum_stash << ") ";
     if (pipelined) notes << "tma-pipelined ";
@@ -2230,19 +2255,20 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
     std::ostringstream src;
     src << "// generated by gaast_b200 codegen: n=" << h.n << " terms=" << h.total_terms << " arith="
         << (g.strict ? "strict" : "fma") << " sum=" << int(opt.with_sum) << " store=" << int(opt.store_out)
-        << " bcast=0x" << std::hex << opt.broadcast_slots << std::dec << (opt.f32 ? " dtype=f32" : "") << "\n// " << notes.str() << "\n";
+        << " bcast=0x" << std::hex << opt.broadcast_slots << std::dec << (opt.f32 ? " dtype=f32" : "") << (opt.wide ? " arith=f64" : "") << "\n// " << notes.str() << "\n";
     // Small kernels are pure streaming: ask for several resident blocks so that ptxas does not
     // trade occupancy for hoisting (cfg2_full: 254 registers without this, 2 blocks per SM).
     const size_t live_regs = live_estimate * size_t(ept);
     // (ptxas treats the hint as a register budget to spend: only give it when it is a tight one)
     // (rolled dense product in f32: 64 left components + a 16 x 16 tile = ~110 registers, 4 blocks per SM)
     const int min_blocks = g.dense_tmem ? 3
-                           : g.dense.op >= 0 ? (opt.f32 ? 4 : (opt.variant & 524288) ? 3 : 1)  // (bit 19: experiment, 168 registers)
-                           : live_regs <= (opt.f32 ? 80u : 40u) ? 8 : live_regs <= (opt.f32 ? 128u : 64u) ? 4 : 1;
+                           : g.dense.op >= 0 ? (cf32 ? 4 : (opt.variant & 524288) ? 3 : 1)  // (bit 19: experiment, 168 registers)
+                           : live_regs <= (cf32 ? 80u : 40u) ? 8 : live_regs <= (cf32 ? 128u : 64u) ? 4 : 1;
     res.min_blocks = min_blocks;
     src << "#define GAAST_EPT " << ept << "\n#define GAAST_THREADS " << threads << "\n#define GAAST_MIN_BLOCKS "
         << min_blocks << "\n";
-    src << kEvalArgsText << "\nusing gaast::EvalArgs;\n" << kPreludeExpLog << (opt.f32 ? kPreludeF32Head : kPrelude) << kPreludeShared << (opt.f32 ? kPreludeF32Tail : kPreludeTail) << "\n";
+    src << kEvalArgsText << "\nusing gaast::EvalArgs;\n" << kPreludeExpLog << (cf32 ? kPreludeF32Head : kPrelude) << kPreludeShared << (cf32 ? kPreludeF32Tail : kPreludeTail)
+        << (opt.wide ? kPreludeWide : "") << "\n";
 
     std::ostringstream loop_strides;
     auto stream_decls = [&](std::ostringstream& o, bool prologue) {
@@ -2282,7 +2308,7 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
         src << "extern \"C\" __global__ void __launch_bounds__(32) gaast_uniform(const __grid_constant__ EvalArgs a) {\n";
         src << "  if (threadIdx.x != 0 || blockIdx.x != 0) return;\n";
         stream_decls(src, true);
-        if (opt.f32) src << "  float* __restrict__ uo = reinterpret_cast<float*>(const_cast<double*>(a.uniform));\n";
+        if (cf32) src << "  float* __restrict__ uo = reinterpret_cast<float*>(const_cast<double*>(a.uniform));\n";
         else src << "  double* __restrict__ uo = const_cast<double*>(a.uniform);\n";
         src << g.body.str();
         for (auto& ex : exports) src << "  uo[" << ex.first << "] = " << g.var(ex.second) << ";\n";
@@ -2321,7 +2347,7 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
         g.body.str("");
         g.indent = 2;
         g.in_loop = true;
-        if (g.n_export > 0 && opt.f32)
+        if (g.n_export > 0 && cf32)
             loop_strides << "    const float* uni = reinterpret_cast<const float*>(a.uniform); asm volatile(\"\" : \"+l\"(uni));\n";
         else if (g.n_export > 0) loop_strides << "    const double* uni = a.uniform; asm volatile(\"\" : \"+l\"(uni));\n";
     }
@@ -2459,7 +2485,7 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
     } else if (tmem_sum) {
         if (n_smem_rows)
             {
-                if (opt.f32) src << "  const unsigned xb = (unsigned)__cvta_generic_to_shared(reinterpret_cast<float*>(sums + " << sum_doubles << ") + tid);\n";
+                if (cf32) src << "  const unsigned xb = (unsigned)__cvta_generic_to_shared(reinterpret_cast<float*>(sums + " << sum_doubles << ") + tid);\n";
                 else src << "  const unsigned xb = (unsigned)__cvta_generic_to_shared(sums + " << sum_doubles << " + tid);\n";
             }
         src << "  const long long n_tiles = (a.n + GAAST_THREADS - 1) / GAAST_THREADS;\n";
@@ -2496,7 +2522,7 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
         std::vector<const Node*> parked(size_t(P), nullptr);
         for (const Node& n : g.nodes)
             if (n.live && n.k == N_LOAD && !n.uniform && n.reload) parked[size_t(n.smem_row)] = &n;
-        if (opt.f32) src << "  float* const stage0 = reinterpret_cast<float*>(sums + " << sum_doubles << ");\n";
+        if (cf32) src << "  float* const stage0 = reinterpret_cast<float*>(sums + " << sum_doubles << ");\n";
         else src << "  double* const stage0 = sums + " << sum_doubles << ";\n";
         src << "  unsigned long long* const stage_bar = reinterpret_cast<unsigned long long*>(stage0 + " << P
             << " * GAAST_THREADS);\n";
@@ -2581,7 +2607,7 @@ static CodegenResult generate(const DevicePlanHost& h, const CodegenOptions& opt
     } else {
         if (n_smem_rows)
             {
-                if (opt.f32) src << "  const unsigned xb = (unsigned)__cvta_generic_to_shared(reinterpret_cast<float*>(sums + " << sum_doubles << ") + tid);\n";
+                if (cf32) src << "  const unsigned xb = (unsigned)__cvta_generic_to_shared(reinterpret_cast<float*>(sums + " << sum_doubles << ") + tid);\n";
                 else src << "  const unsigned xb = (unsigned)__cvta_generic_to_shared(sums + " << sum_doubles << " + tid);\n";
             }
         src << "  for (long long e = ((long long)blockIdx.x * GAAST_THREADS + tid) * GAAST_EPT; e < a.n;\n"

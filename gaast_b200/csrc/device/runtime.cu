@@ -161,7 +161,7 @@ void bind_streams(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_input
 // A batch it cannot address with 128-bit accesses gets one element per thread and no TMA (bulk copies need 16-byte
 // aligned row segments).
 gaast::CodegenOptions specialized_options(const gaast_plan* plan, uint64_t broadcast_slots, int arith, bool with_sum,
-                                          bool store_out, bool f32, const std::vector<std::vector<uint64_t>>& sparse,
+                                          bool store_out, bool f32, bool wide, const std::vector<std::vector<uint64_t>>& sparse,
                                           uint64_t sparse_hash, bool aligned) {
     gaast::CodegenOptions opt;
     opt.broadcast_slots = broadcast_slots;
@@ -169,6 +169,7 @@ gaast::CodegenOptions specialized_options(const gaast_plan* plan, uint64_t broad
     opt.with_sum = with_sum;
     opt.store_out = store_out;
     opt.f32 = f32;
+    opt.wide = wide;
     opt.sparse = sparse;
     opt.sparse_hash = sparse_hash;
     opt.variant = plan->variant;
@@ -177,6 +178,15 @@ gaast::CodegenOptions specialized_options(const gaast_plan* plan, uint64_t broad
     opt.pipelined = aligned && (plan->variant & 8);
     opt.tma_stage = aligned && !opt.pipelined && !with_sum && !(plan->variant & 1024);
     return opt;
+}
+
+// Splits GAAST_ARITH_F64 off an entry point's `arith`: returns GAAST_ARITH_FMA or GAAST_ARITH_STRICT, the only values
+// the engines ever see, and sets *wide when the call evaluates f32 batches in binary64 (the flag means nothing for f64).
+int split_arith(int arith, bool f32, bool* wide) {
+    const int base = arith & ~GAAST_ARITH_F64;
+    if (base != GAAST_ARITH_FMA && base != GAAST_ARITH_STRICT) throw Error(GAAST_ERR_INVALID, "unknown arith mode");
+    *wide = f32 && (arith & GAAST_ARITH_F64) != 0;
+    return base;
 }
 
 // A chain of geometric products runs on the dense engine's matrix-representation kernel unless variant bit 20 asks
@@ -408,9 +418,12 @@ static size_t kernel_source_impl(gaast_plan* plan, uint64_t broadcast_slots, int
                 sparse[i].assign(present[i], present[i] + words);
             }
         }
+        const bool f32 = (with_sum & GAAST_SRC_F32) != 0;
+        bool wide = false;
+        arith = split_arith(arith, f32, &wide);
         // the kernel gaast_eval launches for an aligned batch
-        gaast::CodegenResult cg = gaast::generate_kernel(
-            plan->h, specialized_options(plan, broadcast_slots, arith, sum, store, (with_sum & GAAST_SRC_F32) != 0, sparse, 0, true));
+        gaast::CodegenResult cg =
+            gaast::generate_kernel(plan->h, specialized_options(plan, broadcast_slots, arith, sum, store, f32, wide, sparse, 0, true));
         len = cg.source.size();
         if (buf && cap) {
             const size_t ncopy = std::min(cap - 1, len);
@@ -440,8 +453,10 @@ gaast_status gaast_plan_precompile_typed(gaast_plan* plan, uint64_t broadcast_sl
     return guard([&] {
         if (!plan) throw Error(GAAST_ERR_INVALID, "null plan");
         const bool f32 = dtype == GAAST_F32;
+        bool wide = false;
+        arith = split_arith(arith, f32, &wide);
         auto options = [&](bool aligned) {
-            return specialized_options(plan, broadcast_slots, arith, with_sum != 0, store_out != 0, f32, {}, 0, aligned);
+            return specialized_options(plan, broadcast_slots, arith, with_sum != 0, store_out != 0, f32, wide, {}, 0, aligned);
         };
         gaast::CodegenResult cg;
         std::string key, origin;
@@ -916,8 +931,9 @@ static std::shared_ptr<gaast::JitKernel> dense_kernel(gaast_plan* plan, long lon
 struct EvalCall {
     gaast_plan* plan;
     gaast_batch* out;  // null: sums only
-    int arith;
+    int arith;  // GAAST_ARITH_FMA or GAAST_ARITH_STRICT (split_arith)
     bool with_sum, f32 = false;
+    bool wide = false;  // f32 batches evaluated in binary64
     gaast::EvalArgs a{};
     uint64_t bslots = 0;  // broadcast input slots
     long long n = 0;
@@ -1004,7 +1020,7 @@ static Engine choose_engine(EvalCall& c, int engine, std::shared_ptr<gaast::JitK
     c.n = c.a.n = len.n;
     try {
         *jk = get_specialized(c.plan, specialized_options(c.plan, c.bslots, c.arith, c.with_sum, c.out != nullptr, c.f32,
-                                                          c.sparse, c.sparse_hash, len.aligned));
+                                                          c.wide, c.sparse, c.sparse_hash, len.aligned));
         return Engine::specialized;
     } catch (const Error&) {
         // AUTO: this variant cannot be specialised (too large, or no NVRTC and no cached cubin): another engine
@@ -1161,7 +1177,7 @@ static int launch_specialized(EvalCall& c, const gaast::JitKernel& jk) {
 static int launch_table(EvalCall& c) {
     gaast_plan* plan = c.plan;
     gaast_ctx* ctx = plan->ctx;
-    const gaast::TableLaunch shape = gaast::table_engine_shape(*ctx, plan->h, c.n, c.with_sum, c.f32);
+    const gaast::TableLaunch shape = gaast::table_engine_shape(*ctx, plan->h, c.n, c.with_sum, c.f32, c.wide);
     // scratch is sized for the largest grid the engine ever launches (8 blocks per SM)
     const size_t max_grid = std::max(size_t(shape.grid), size_t(ctx->sm_count) * 8);
     if (shape.global_ws) {
@@ -1173,7 +1189,7 @@ static int launch_table(EvalCall& c) {
     c.a.chunks = plan->d_chunks;
     c.a.n_micro = int(plan->h.micro.size());
     c.a.n_chunks = int(plan->h.chunks.size());
-    cuda_check(gaast::table_engine_launch(c.a, shape, c.arith == GAAST_ARITH_STRICT, c.with_sum, c.f32, ctx->stream),
+    cuda_check(gaast::table_engine_launch(c.a, shape, c.arith == GAAST_ARITH_STRICT, c.with_sum, c.f32, c.wide, ctx->stream),
                "launch table engine");
     ctx->launches++;
     char desc[256];
@@ -1188,13 +1204,15 @@ static void eval_impl(gaast_plan* plan, gaast_batch* const* inputs, uint32_t n_i
     if (!plan) throw Error(GAAST_ERR_INVALID, "null plan");
     gaast_ctx* ctx = plan->ctx;
     if (!ctx) throw Error(GAAST_ERR_NO_DEVICE, "this plan was created without a ctx (offline): it cannot be evaluated");
-    if (arith != GAAST_ARITH_FMA && arith != GAAST_ARITH_STRICT) throw Error(GAAST_ERR_INVALID, "unknown arith mode");
+    bool wide = false;
+    split_arith(arith, false, &wide);  // (unknown bits are refused before the batches are looked at)
     if (with_sum && !dev_sum) throw Error(GAAST_ERR_INVALID, "eval_sum: null sum pointer");
     DeviceGuard dg(ctx->device);
     EvalCall c{plan, out, arith, with_sum};
     int dtype = GAAST_F64;
     bind_streams(plan, inputs, n_inputs, out, !with_sum, c.a, &c.bslots, &c.n, &dtype, &c.sparse, &c.sparse_hash);
     c.f32 = dtype == GAAST_F32;
+    c.arith = split_arith(arith, c.f32, &c.wide);
     if (!c.sparse.empty() && (engine == GAAST_ENGINE_TABLE || engine == GAAST_ENGINE_DENSE_WARP))
         throw Error(GAAST_ERR_UNSUPPORTED, "sparse batches are evaluated by the specialised engine only (the kernel is "
                                            "generated for the sparsity pattern): use GAAST_ENGINE_AUTO or GAAST_ENGINE_SPECIALIZED");

@@ -102,9 +102,10 @@ __device__ __forceinline__ T log_factor(T a0, T q) {
 // kGlobalWs is a template parameter so that, in the common case, the compiler knows the
 // workspace is shared memory and emits LDS/STS instead of generic loads and stores.
 constexpr int kLanes = 32;
-// T = scalar type of the batches and of the workspace (double, or float for the f32 variant);
-// the batch-sum columns are double in both cases and follow the T workspace.
-template <class T, bool kStrict, bool kSum, bool kGlobalWs>
+// T = scalar type of the arithmetic and of the workspace (double, or float for the f32 variant), St = scalar type of the
+// batches (float for f32 batches, also when they are evaluated in double: loads widen, stores round once);
+// the batch-sum columns are double in every case, add the unrounded T results and follow the T workspace.
+template <class T, bool kStrict, bool kSum, bool kGlobalWs, class St = T>
 __global__ void __launch_bounds__(256) table_engine_kernel(const __grid_constant__ EvalArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     TermChunk* stage = reinterpret_cast<TermChunk*>(smem_raw);
@@ -152,11 +153,11 @@ __global__ void __launch_bounds__(256) table_engine_kernel(const __grid_constant
             switch (op.kind) {
                 case MK_LOAD_ADD: {  // eval.rs:45-50
                     const bool bc = (a.bcast[op.a >> 6] >> (op.a & 63)) & 1;
-                    const T* src = reinterpret_cast<const T*>(a.sptr[op.a]) + (long long)op.b * a.srow[op.a] + (bc ? 0 : e);
+                    const St* src = reinterpret_cast<const St*>(a.sptr[op.a]) + (long long)op.b * a.srow[op.a] + (bc ? 0 : e);
                     const long long rs = a.srow[op.a];
                     for (uint32_t r = grp; r < op.count; r += G) {
                         T* d = &w[size_t(op.dst_col + r) * kLanes];
-                        const T v = active ? __ldg(src + r * rs) : T(0);
+                        const T v = active ? T(__ldg(src + r * rs)) : T(0);
                         *d = kStrict ? add_rn(*d, v) : (*d + v);
                     }
                     break;
@@ -248,11 +249,11 @@ __global__ void __launch_bounds__(256) table_engine_kernel(const __grid_constant
                     }
                     break;
                 case MK_STORE: {
-                    T* dst = reinterpret_cast<T*>(a.sptr[op.a]) + (long long)op.b * a.srow[op.a] + e;
+                    St* dst = reinterpret_cast<St*>(a.sptr[op.a]) + (long long)op.b * a.srow[op.a] + e;
                     const long long rs = a.srow[op.a];
                     for (uint32_t r = grp; r < op.count; r += G) {
                         const T v = w[size_t(op.dst_col + r) * kLanes];
-                        if (active && a.store_out) dst[r * rs] = v;
+                        if (active && a.store_out) dst[r * rs] = St(v);  // (double -> float: round to nearest even)
                         if (kSum && active) {
                             double* sc = &sw[size_t(op.pad0 + r) * kLanes];  // (pad0: the run's first batch-sum column)
                             *sc = *sc + double(v);
@@ -322,32 +323,38 @@ __global__ void reduce_partials_stage1(const double* __restrict__ partials, int 
     }
 }
 
+// T = Scalars<arithmetic type, batch type> (below)
 template <class T, bool kStrict, bool kSum, bool kGlobalWs>
 cudaError_t launch_g(const EvalArgs& args, const TableLaunch& shape, cudaStream_t stream) {
-    auto k = table_engine_kernel<T, kStrict, kSum, kGlobalWs>;
+    auto k = table_engine_kernel<typename T::compute, kStrict, kSum, kGlobalWs, typename T::storage>;
     cudaError_t err = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, int(shape.smem));
     if (err != cudaSuccess) return err;
     k<<<shape.grid, shape.threads, shape.smem, stream>>>(args);
     return cudaGetLastError();
 }
-template <class T, bool kStrict, bool kSum>
+template <class T, class St>
+struct Scalars {
+    using compute = T;
+    using storage = St;
+};
+template <class T, class St, bool kStrict, bool kSum>
 cudaError_t launch_t(const EvalArgs& args, const TableLaunch& shape, cudaStream_t stream) {
-    return shape.global_ws ? launch_g<T, kStrict, kSum, true>(args, shape, stream)
-                           : launch_g<T, kStrict, kSum, false>(args, shape, stream);
+    return shape.global_ws ? launch_g<Scalars<T, St>, kStrict, kSum, true>(args, shape, stream)
+                           : launch_g<Scalars<T, St>, kStrict, kSum, false>(args, shape, stream);
 }
-template <class T>
+template <class T, class St>
 cudaError_t launch_s(const EvalArgs& args, const TableLaunch& shape, bool strict, bool with_sum, cudaStream_t stream) {
-    if (strict) return with_sum ? launch_t<T, true, true>(args, shape, stream) : launch_t<T, true, false>(args, shape, stream);
-    return with_sum ? launch_t<T, false, true>(args, shape, stream) : launch_t<T, false, false>(args, shape, stream);
+    if (strict) return with_sum ? launch_t<T, St, true, true>(args, shape, stream) : launch_t<T, St, true, false>(args, shape, stream);
+    return with_sum ? launch_t<T, St, false, true>(args, shape, stream) : launch_t<T, St, false, false>(args, shape, stream);
 }
 
 }  // namespace
 
-TableLaunch table_engine_shape(const gaast_ctx& ctx, const DevicePlanHost& h, long long n, bool with_sum, bool f32) {
+TableLaunch table_engine_shape(const gaast_ctx& ctx, const DevicePlanHost& h, long long n, bool with_sum, bool f32, bool wide) {
     TableLaunch s;
     const size_t cols = h.total_cols + (with_sum ? h.stored_cols : 0);
-    // one tile = 32 elements; the sum columns are doubles in both variants
-    const size_t ws_bytes = (h.total_cols * (f32 ? sizeof(float) : sizeof(double)) + (with_sum ? h.stored_cols * sizeof(double) : 0)) * kLanes;
+    // one tile = 32 elements; the workspace holds the arithmetic's type, the sum columns are doubles in every variant
+    const size_t ws_bytes = (h.total_cols * (f32 && !wide ? sizeof(float) : sizeof(double)) + (with_sum ? h.stored_cols * sizeof(double) : 0)) * kLanes;
     s.threads = 256;                                         // 8 warps share the tile's work
     s.global_ws = kWsOffset + ws_bytes > size_t(ctx.smem_optin);
     s.smem = s.global_ws ? kWsOffset : kWsOffset + ws_bytes;
@@ -361,8 +368,10 @@ TableLaunch table_engine_shape(const gaast_ctx& ctx, const DevicePlanHost& h, lo
 }
 
 cudaError_t table_engine_launch(const EvalArgs& args, const TableLaunch& shape, bool strict, bool with_sum, bool f32,
-                                cudaStream_t stream) {
-    return f32 ? launch_s<float>(args, shape, strict, with_sum, stream) : launch_s<double>(args, shape, strict, with_sum, stream);
+                                bool wide, cudaStream_t stream) {
+    if (f32 && wide) return launch_s<double, float>(args, shape, strict, with_sum, stream);
+    return f32 ? launch_s<float, float>(args, shape, strict, with_sum, stream)
+               : launch_s<double, double>(args, shape, strict, with_sum, stream);
 }
 
 cudaError_t reduce_partials_launch(const double* partials, int n_blocks, int n_cols, double* out,

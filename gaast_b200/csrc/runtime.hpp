@@ -48,6 +48,7 @@ struct CodegenOptions {
     bool tma_stage = false;    // one-tile blocks: parked rows copied to shared memory by TMA bulk copies (aligned rows)
     int extra_parked = 0;      // more input rows parked in shared memory (raised while ptxas reports spills)
     bool f32 = false;          // binary32 batches and arithmetic (the f32 variant); batch sums stay in double
+    bool wide = false;         // with f32: binary64 arithmetic on the binary32 batches (GAAST_ARITH_F64), one rounding per store
     // Sparse per-grade storage of the bound inputs: per stream (device_plan.hpp) a bitmap of the components its grade
     // array stores (empty = dense).  Components that are not stored are zero for every element: their loads become
     // the constant 0 and every term that reads them is dropped (exactly, in strict arithmetic too: x + 0 * y == x
@@ -57,7 +58,7 @@ struct CodegenOptions {
     // What tells two specialised kernels of one plan apart (the bitmaps by their hash): the plan's map key.
     auto key() const {
         return std::make_tuple(broadcast_slots, arith, with_sum, store_out, elems_per_thread, variant, pipelined, tma_stage,
-                               f32, sparse_hash);
+                               f32, wide, sparse_hash);
     }
 };
 
@@ -102,9 +103,10 @@ struct TableLaunch {
     bool global_ws = false;
     size_t ws_doubles_per_block = 0;  // global workspace: columns x 32 lanes
 };
-TableLaunch table_engine_shape(const gaast_ctx& ctx, const DevicePlanHost& h, long long n, bool with_sum, bool f32);
+// f32: binary32 batches; wide: evaluated in binary64 (the workspace is then sized in doubles)
+TableLaunch table_engine_shape(const gaast_ctx& ctx, const DevicePlanHost& h, long long n, bool with_sum, bool f32, bool wide);
 cudaError_t table_engine_launch(const EvalArgs& args, const TableLaunch& shape, bool strict, bool with_sum, bool f32,
-                                cudaStream_t stream);
+                                bool wide, cudaStream_t stream);
 // (the partials buffer must have room for kReduceStage1Rows more rows of n_cols doubles: the two-level reduction's scratch)
 constexpr int kReduceStage1Rows = 296;
 cudaError_t reduce_partials_launch(const double* partials, int n_blocks, int n_cols, double* out,

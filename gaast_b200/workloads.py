@@ -220,6 +220,10 @@ def precompile_variants(w: Workload):
     variants += [(L.ARITH_FMA, False, True, L.F32), (L.ARITH_STRICT, False, True, L.F32)]
     if w.sum_root:
         variants += [(L.ARITH_FMA, True, True, L.F32)]
+    # f32 batches evaluated in binary64 (tests/test_gpu_f32_wide.py, tools/f32_wide_bw.py)
+    variants += [(L.ARITH_FMA | L.ARITH_F64, False, True, L.F32)]
+    if w.sum_root:
+        variants += [(L.ARITH_FMA | L.ARITH_F64, True, True, L.F32)]
     return variants
 
 
@@ -239,7 +243,8 @@ def precompile_all(verbose: bool = False, fresh: bool = True) -> int:
             info = plan.precompile(w.broadcast_mask(), arith, with_sum, store, dtype)
             count += 1
             if verbose:
-                print(f"  {w.name:10s} {'f32' if dtype else 'f64'} arith={'strict' if arith else 'fma':6s} sum={int(with_sum)} "
+                mode = ('strict' if arith & L.ARITH_STRICT else 'fma') + ('|f64' if arith & L.ARITH_F64 else '')
+                print(f"  {w.name:10s} {'f32' if dtype else 'f64'} arith={mode:6s} sum={int(with_sum)} "
                       f"store={int(store)}: {info}")
         plan.free()
     # bench.py also times cfg3 / cfg5 with their algebraic lowering switched off (variant bits 17 / 16)

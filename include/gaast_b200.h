@@ -165,12 +165,23 @@ typedef enum gaast_arith {
     GAAST_ARITH_FMA = 0,   /* one DFMA per term (default; within 1e-12 of eval.rs) */
     GAAST_ARITH_STRICT = 1 /* (l*r)*coeff then add, reference order: bit-identical to eval.rs */
 } gaast_arith;
+/* A flag OR-ed into `arith` (GAAST_ARITH_FMA | GAAST_ARITH_F64, GAAST_ARITH_STRICT | GAAST_ARITH_F64): f32 batches
+ * evaluated in binary64.  Every load is widened to binary64, all arithmetic (products, sign flips, 1/x, sqrt, exp / log,
+ * hoisted linear-map coefficients) is binary64, plan literals and term coefficients stay binary64, and each stored
+ * result is rounded ONCE to binary32, to nearest even.  STRICT | F64 is bit-identical to float32(eval.rs evaluated on
+ * the widened inputs); FMA | F64 is within 1e-12 of max(|ref|, sum |terms|) before that rounding.  Batch sums
+ * (gaast_eval_sum) add the unrounded binary64 results, not the stored binary32 values: they are held to the f64 bar.
+ * The HBM bytes are the f32 variant's (gaast_plan_cost counts storage bytes).  On f64 batches the flag changes
+ * nothing: same kernel, same bits.  GAAST_ENGINE_DENSE_WARP is GAAST_ERR_UNSUPPORTED for f32 batches with or without
+ * it; any other bit in `arith` is GAAST_ERR_INVALID. */
+#define GAAST_ARITH_F64 2
 
 /* Scalar type of a batch.  f64 is the reference's type (eval.rs works on f64 only) and the
  * type every parity claim is made in.  f32 is this library's reduced-precision variant
  * (SURVEY.md 8f rank 4): the same plans evaluated in IEEE binary32 -- half the HBM bytes.
  * All batches of one gaast_eval call must share one dtype; plan literals and term
- * coefficients are rounded to binary32; batch sums still accumulate in f64. */
+ * coefficients are rounded to binary32; batch sums still accumulate in f64.  GAAST_ARITH_F64
+ * keeps the f32 storage and evaluates in binary64 instead. */
 typedef enum gaast_dtype {
     GAAST_F64 = 0,
     GAAST_F32 = 1
@@ -235,7 +246,8 @@ uint32_t gaast_plan_slot_mask(const gaast_plan* plan, uint32_t slot);
  * nvcc -Xptxas -v / the CPU run of the generated text in tests/kernel_emu); returns the length, copies at most `cap`
  * bytes (NUL-terminated).  `with_sum` is a set of GAAST_SRC_* flags: 0 / 1 keep their meaning (plain kernel / fused
  * batch-sum); GAAST_SRC_NO_STORE = the kernel gaast_eval_sum launches with out == NULL (sums only),
- * GAAST_SRC_F32 = the kernel of the f32 variant. */
+ * GAAST_SRC_F32 = the kernel of the f32 variant (with `arith` | GAAST_ARITH_F64: the f32 kernel in binary64
+ * arithmetic; without GAAST_SRC_F32 the flag changes nothing). */
 #define GAAST_SRC_WITH_SUM 1
 #define GAAST_SRC_NO_STORE 2
 #define GAAST_SRC_F32 4
@@ -403,7 +415,8 @@ gaast_status gaast_eval_host(gaast_plan* plan, const double* const* host_in, con
                              const int* in_broadcast, uint32_t n_inputs, uint64_t len, uint64_t host_stride,
                              double* host_out, int engine, int arith);
 
-/* The same pipeline for binary32 host arrays (the f32 variant; half the PCIe traffic). */
+/* The same pipeline for binary32 host arrays (the f32 variant; half the PCIe traffic).  `arith` is passed to
+ * gaast_eval as given: GAAST_ARITH_F64 evaluates the chunks in binary64. */
 gaast_status gaast_eval_host_f32(gaast_plan* plan, const float* const* host_in, const uint32_t* in_masks,
                                  const int* in_broadcast, uint32_t n_inputs, uint64_t len, uint64_t host_stride,
                                  float* host_out, int engine, int arith);

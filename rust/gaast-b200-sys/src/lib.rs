@@ -43,6 +43,8 @@ pub const GAAST_ENGINE_SPECIALIZED: c_int = 2;
 pub const GAAST_ENGINE_DENSE_WARP: c_int = 3;
 pub const GAAST_ARITH_FMA: c_int = 0;
 pub const GAAST_ARITH_STRICT: c_int = 1;
+// OR-ed into `arith`: f32 batches evaluated in binary64, each stored result rounded once
+pub const GAAST_ARITH_F64: c_int = 2;
 pub const GAAST_F64: c_int = 0;
 pub const GAAST_F32: c_int = 1;
 pub const GAAST_HOST_DEFAULT: c_int = 0;
